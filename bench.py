@@ -236,13 +236,13 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), last
 
     parity = None
     if rank == 0 and not args.no_parity and args.path == "fused":
@@ -256,8 +256,17 @@ def run_ours(args):
     for _ in range(400):                  # ~1 s more under load on EVERY rank (the step holds a collective), so
         device_step()                     # that the sampler has several readings under load before the clock starts
     l0 = _lib.launch_count()
-    ms = timed(device_step, args.steps)
+    ms, last_loss = timed(device_step, args.steps)
     launches = _lib.launch_count() - l0
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step holds after the last timed step: its loss, the gradients it wrote and the
+        # parameters Adam updated (copied now: the steps below overwrite all three)
+        dump = {"loss": last_loss.detach().reshape(1).cpu()}
+        for n, p in model.named_parameters():
+            if p.requires_grad:
+                dump["grad." + n] = p.grad.detach().cpu()
+                dump["param." + n] = p.detach().cpu()
     if sampler:
         sampler.stop_flag = True
     for _ in range(2):
@@ -298,7 +307,7 @@ def run_ours(args):
     # acquisition slice (C5-shaped): n candidates x S=25 samples through an (uncond, cond) pair at the top fidelity
     acq = None
     if not args.no_acq:
-        acq = bench_acq(model, dev, cfg, world, rank, n=args.acq_candidates, with_cpu=not args.no_cpu)
+        acq = bench_acq(model, dev, cfg, world, rank, n=args.acq_candidates, with_cpu=not args.no_cpu, dump=dump)
 
     if rank == 0:
         flops, f1 = step_flops(cfg)
@@ -366,9 +375,34 @@ def run_ours(args):
             out["small_configs"] = bench_small_configs(dev)
         if not args.no_cpu and world == 1:      # reported on rank 0 at N = 1 only
             out["cpu_baseline"] = cpu_baseline(cfg, x, y, fid, model, steps=8, warmup=2)
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_SAMPLE = 1 << 20          # entries kept of a larger output array
+DUMP_MAX_BYTES = 64 << 20
+
+
+def write_outputs(directory, arrays):
+    """``--dump-outputs``: every array as ``directory/<name>.npy`` in float64.  An array of more than DUMP_SAMPLE
+    entries is flattened and reduced to the entries at DUMP_SAMPLE positions drawn with a fixed seed, so that runs with
+    the same arguments write the same positions and two builds can be compared entry for entry."""
+    import numpy as np
+    out = {}
+    for name, t in arrays.items():
+        a = t.double().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        out[name] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def bench_small_configs(dev, steps=200):
@@ -660,7 +694,8 @@ def acq_flop_per_candidate(cfg, K, P, S=25):
     return K * (1 + P) * (f0 + (L - 1) * S * f1)
 
 
-def bench_acq(model, dev, cfg, world, rank, n=C5_CANDIDATES_PER_GPU, K=6, P=16, iters=1, with_cpu=True, n_grad=1024):
+def bench_acq(model, dev, cfg, world, rank, n=C5_CANDIDATES_PER_GPU, K=6, P=16, iters=1, with_cpu=True, n_grad=1024,
+              dump=None):
     """JESMOC acquisition sweep, BASELINE.json configs[4] (SURVEY.md section 8d "C5"): every rank evaluates ITS n
     candidates (10^6 over 8 GPUs = 125 000 per GPU; candidates shard, no data-path collective) through the full coupled
     acquisition: K = 6 black boxes (4 objectives + 2 constraints) x (1 unconditioned + P = 16 Pareto-conditioned) MFDGPs
@@ -670,7 +705,7 @@ def bench_acq(model, dev, cfg, world, rank, n=C5_CANDIDATES_PER_GPU, K=6, P=16, 
     (mobocmf/acquisition_functions/JESMOC_MFDGP.py:38-52,125-135; mobocmf_b200...JESMOC_MFDGP.jes_sweep).  One 'eval'
     = one candidate through all 102 chains.  Legs: device-resident forward (value), end to end from pinned host
     memory (e2e), forward + d/dX on n_grad candidates (what optimize_acqf consumes), the CPU oracle on a bounded slice
-    (rank 0, N = 1)."""
+    (rank 0, N = 1).  ``dump``: a dict that receives the values of the timed sweep."""
     import torch.distributed as dist
     from mobocmf_b200.acquisition_functions.JESMOC_MFDGP import jes_sweep
     fidelity = cfg["L"] - 1
@@ -699,6 +734,8 @@ def bench_acq(model, dev, cfg, world, rank, n=C5_CANDIDATES_PER_GPU, K=6, P=16, 
     e1.record()
     barrier()
     ms = sync_max(e0.elapsed_time(e1) / iters)
+    if dump is not None:
+        dump["acq_values"] = out.cpu()
 
     # end to end: candidates from pinned host memory, values back to pinned host memory, host waits for them
     vals_h = torch.empty(n, dtype=torch.float64).pin_memory()
@@ -975,7 +1012,14 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the CUDA-vs-oracle parity block")
     ap.add_argument("--acq-candidates", type=int, default=C5_CANDIDATES_PER_GPU,
                     help="candidates per GPU of the C5 acquisition sweep (10^6 / 8 by default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, gradients, updated parameters) and the values "
+                         "of the timed acquisition sweep as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
