@@ -32,7 +32,9 @@
 extern "C" {
 #endif
 
-/* library / build identification: 102 (sm_100a; 100 + ABI revision; 2: mobo_step_desc.ctx, step contexts) */
+/* library / build identification: 103 (sm_100a; 100 + ABI revision; 2: mobo_step_desc.ctx, step contexts;
+ * 3: the multi-layer operator-chain entry points and the stand-alone K(Z, Z) entry point removed, more scratch for
+ * mobo_layer_rows_bwd) */
 int mobo_abi_version(void);
 
 /* Launch accounting: number of kernels this library has launched in this process; optional per-launch CUDA-event
@@ -58,17 +60,6 @@ size_t mobo_precompute_bwd_work_doubles(int M);
  * m: M variational mean; Lq: M x M chol_variational_covar (tril applied inside). */
 int mobo_layer_precompute(int kind, int d, int M, const double* Zx, const double* zf, const double* theta,
                           const double* m, const double* Lq, double jitter, double* ops, void* stream);
-
-/* The same for all layers of a model in one batch of launches (the layers' operator chains are independent).
- * Arrays of length nl (HOST arrays of device pointers); zf[i] is NULL for kind 0. */
-int mobo_model_precompute(int nl, const int* kinds, int d, int M, const double* const* Zx, const double* const* zf,
-                          const double* const* theta, const double* const* m, const double* const* Lq,
-                          double jitter, double* const* ops, void* stream);
-int mobo_model_precompute_bwd(int nl, const int* kinds, int d, int M, const double* const* Zx,
-                              const double* const* zf, const double* const* theta, const double* const* m,
-                              const double* const* Lq, const double* const* ops, const double* const* gops,
-                              double* const* work, double* const* dtheta, double* const* dzf, double* const* dm,
-                              double* const* dLq, void* stream);
 
 /* Backward of mobo_layer_precompute.  gops: gradient buffer (convention above).  work:
  * mobo_precompute_bwd_work_doubles(M).  Outputs: dtheta[theta size], dzf[M] (kind 1), dm[M], dLq[M x M]. */
@@ -102,10 +93,6 @@ int mobo_layer_rows_bwd(int kind, int d, int M, const double* Zx, const double* 
                         const unsigned int* clamp_count, const double* Tsave,
                         const double* Usave, int want_param_grads, double* df, double* dxrow, double* dtheta,
                         double* dzf, double* gops, double* work, void* stream);
-
-/* Dense K(Z_l, Z_l) + jitter I into P (MP x MP) — exposed for tests. */
-int mobo_kzz(int kind, int d, int M, const double* Zx, const double* zf, const double* theta, double jitter,
-             double* P, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Fused ELBO step: the body of BlackBoxMFDGPFitter._update_model up to the gradients

@@ -27,11 +27,8 @@ _SIGNATURES = {
     "mobo_rows_save_doubles": (_c_sz, [_c_i, _c_ll]),
     "mobo_rows_bwd_work_doubles": (_c_sz, [_c_i, _c_ll]),
     "mobo_precompute_bwd_work_doubles": (_c_sz, [_c_i]),
-    "mobo_kzz": (_c_i, [_c_i, _c_i, _c_i, _c_dp, _c_dp, _c_dp, _c_d, _c_dp, _c_dp]),
     "mobo_layer_precompute": (_c_i, [_c_i, _c_i, _c_i, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_d, _c_dp, _c_dp]),
     "mobo_layer_precompute_bwd": (_c_i, [_c_i, _c_i, _c_i] + [_c_dp] * 13),
-    "mobo_model_precompute": (_c_i, [_c_i, _c_dp, _c_i, _c_i, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_d, _c_dp, _c_dp]),
-    "mobo_model_precompute_bwd": (_c_i, [_c_i, _c_dp, _c_i, _c_i] + [_c_dp] * 13),
     "mobo_layer_rows_fwd": (_c_i, [_c_i, _c_i, _c_i, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_i, _c_dp, _c_dp, _c_i,
                                    _c_dp, _c_ll, _c_dp, _c_ll, _c_i, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp,
                                    _c_dp]),

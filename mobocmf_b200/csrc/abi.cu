@@ -12,12 +12,14 @@
 
 using namespace mobo;
 
+static_assert(kMaxLayers == MOBO_MAX_LAYERS && kMaxTheta == MOBO_MAX_THETA, "the kernels' limits are the header's");
+
 static inline int padded(int M) { return ((M + 31) / 32) * 32; }
 #define MOBO_TRY(x) do { int _e = (x); if (_e) return _e; } while (0)
 
 extern "C" {
 
-int mobo_abi_version(void) { return 102; }
+int mobo_abi_version(void) { return 103; }
 
 long long mobo_launch_count(void) { return prof_state().launches; }
 
@@ -55,65 +57,29 @@ size_t mobo_rows_save_doubles(int M, long long R) {
 
 size_t mobo_rows_bwd_work_doubles(int M, long long R) {
   const int MP = padded(M);
-  return (size_t)256 * KG_CTAS_PER_SM * (MAX_THETA + MP) + syrk_part_doubles(MP, R) + syrk_alpha_doubles(MP, syrk_nchunk(MP, R)) + 64 +
-         mobo_rows_save_doubles(M, R);   // + the dk scratch [R][MP]
+  return (size_t)256 * KG_CTAS_PER_SM * (kMaxTheta + MP) + 2 * syrk_part_doubles(MP, R) +
+         syrk_alpha_doubles(MP, syrk_nchunk(MP, R)) + 64 + mobo_rows_save_doubles(M, R);   // + the dk scratch [R][MP]
 }
 
 size_t mobo_precompute_bwd_work_doubles(int M) {
   const int MP = padded(M);
-  return (size_t)8 * MP * MP + (size_t)((M + KZB_WARPS - 1) / KZB_WARPS) * KZB_NTH + 64;
+  return (size_t)8 * MP * MP + (size_t)((M + KZB_WARPS - 1) / KZB_WARPS) * kMaxTheta + 64;
 }
 
-static int fill_batch(LayerBatch& b, int nl, const int* kinds, int d, int M, const double* const* Zx,
-                      const double* const* zf, const double* const* theta, const double* const* m,
-                      const double* const* Lq, double* const* ops) {
-  if (nl < 1 || nl > MAX_BATCH) return -2;
-  b.n = nl; b.d = d; b.M = M; b.MP = padded(M);
-  if (d > kMaxD || b.MP > MAX_MP) return -2;
-  for (int i = 0; i < MAX_BATCH; ++i) {
-    const bool ok = i < nl;
-    b.kind[i] = ok ? kinds[i] : 0;
-    b.Zx[i] = ok ? Zx[i] : nullptr;
-    b.zf[i] = (ok && zf) ? zf[i] : nullptr;
-    b.theta[i] = ok ? theta[i] : nullptr;
-    b.m[i] = (ok && m) ? m[i] : nullptr;
-    b.Lq[i] = (ok && Lq) ? Lq[i] : nullptr;
-    b.ops[i] = (ok && ops) ? ops[i] : nullptr;
-  }
-  return 0;
-}
-
-int mobo_kzz(int kind, int d, int M, const double* Zx, const double* zf, const double* theta, double jitter,
-             double* P, void* stream) {
-  // P is written where block OPS_P of an operator buffer starting at (P - OPS_P * MP^2) would live
-  LayerBatch b;
+// The operator chains of nl layers in one cooperative launch: a CTA per 32 x 32 block of the lower triangle of every
+// layer (opchain.cu).  reset_flags = false: the caller has already zeroed the flags region of every operator buffer
+// on this stream.
+static int model_precompute(int nl, const int* kinds, int d, int M, const double* const* Zx, const double* const* zf,
+                            const double* const* theta, const double* const* m, const double* const* Lq,
+                            double jitter, double* const* ops, cudaStream_t st, bool reset_flags) {
   const int MP = padded(M);
-  double* fake_ops = P - ops_block(MP, OPS_P);
-  MOBO_TRY(fill_batch(b, 1, &kind, d, M, &Zx, &zf, &theta, nullptr, nullptr, &fake_ops));
-  cudaStream_t st = (cudaStream_t)stream;
-  MOBO_LAUNCH("kzz_kernel", st, kzz_kernel<<<dim3((MP * MP + 255) / 256, 1), 256, 0, st>>>(b, jitter, OPS_P, 0));
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
-}
-
-static int model_precompute(int nl, const int* kinds, int d, int M, const double* const* Zx, const double* const* zf,
-                            const double* const* theta, const double* const* m, const double* const* Lq,
-                            double jitter, double* const* ops, void* stream, bool reset_flags);
-
-int mobo_model_precompute(int nl, const int* kinds, int d, int M, const double* const* Zx, const double* const* zf,
-                          const double* const* theta, const double* const* m, const double* const* Lq,
-                          double jitter, double* const* ops, void* stream) {
-  return model_precompute(nl, kinds, d, M, Zx, zf, theta, m, Lq, jitter, ops, stream, true);
-}
-
-// reset_flags = false: the caller has already zeroed the flags region of every operator buffer on this stream
-static int model_precompute(int nl, const int* kinds, int d, int M, const double* const* Zx, const double* const* zf,
-                            const double* const* theta, const double* const* m, const double* const* Lq,
-                            double jitter, double* const* ops, void* stream, bool reset_flags) {
-  cudaStream_t st = (cudaStream_t)stream;
-  LayerBatch b;
-  MOBO_TRY(fill_batch(b, nl, kinds, d, M, Zx, zf, theta, m, Lq, ops));
-  const int MP = b.MP;
-  // one cooperative launch: a CTA per 32 x 32 block of the lower triangle of every layer (opchain.cu)
+  if (nl < 1 || nl > kMaxLayers || d > kMaxD || MP > MAX_MP) return -2;
+  LayerBatch b = {};
+  b.n = nl; b.d = d; b.M = M; b.MP = MP;
+  for (int i = 0; i < nl; ++i) {
+    b.kind[i] = kinds[i]; b.Zx[i] = Zx[i]; b.zf[i] = zf[i]; b.theta[i] = theta[i];
+    b.m[i] = m[i]; b.Lq[i] = Lq[i]; b.ops[i] = ops[i];
+  }
   const int nb = MP / 32, nblk = nb * (nb + 1) / 2;
   if (reset_flags) MOBO_LAUNCH("opchain_reset_kernel", st, opchain_reset_kernel<<<nl, 128, 0, st>>>(b));
   void* args[] = {(void*)&b, (void*)&jitter};
@@ -125,122 +91,61 @@ static int model_precompute(int nl, const int* kinds, int d, int M, const double
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
-int mobo_model_precompute_bwd(int nl, const int* kinds, int d, int M, const double* const* Zx,
-                              const double* const* zf, const double* const* theta, const double* const* m,
-                              const double* const* Lq, const double* const* ops, const double* const* gops,
-                              double* const* work, double* const* dtheta, double* const* dzf, double* const* dm,
-                              double* const* dLq, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  LayerBatch b;
-  MOBO_TRY(fill_batch(b, nl, kinds, d, M, Zx, zf, theta, m, Lq, const_cast<double* const*>(ops)));
-  const int MP = b.MP;
-  const size_t MP2 = (size_t)MP * MP;
-  enum { T_G2 = 0, T_V, T_NN, T_F, T_X1, T_DP, T_X2, T_Y2, T_N };
-  auto blk = [&](int i, int which) { return work[i] + (size_t)which * MP2; };
-  auto mk = [&](GemmOperand& o, bool trans, int tri, auto getter) {
-    o.trans = trans; o.tri = tri;
-    for (int i = 0; i < MAX_BATCH; ++i) o.p[i] = i < nl ? getter(i) : nullptr;
-  };
-  double* C[MAX_BATCH];
-  auto outs = [&](int which) { for (int i = 0; i < MAX_BATCH; ++i) C[i] = i < nl ? blk(i, which) : nullptr; };
-  GemmOperand A, B;
-  // G2 = H H^T
-  mk(A, false, 1, [&](int i) { return ops[i] + ops_block(MP, OPS_H); });
-  mk(B, true, 2, [&](int i) { return ops[i] + ops_block(MP, OPS_H); });
-  outs(T_G2);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  // V = A2 G2
-  mk(A, false, 0, [&](int i) { return gops[i] + ops_block(MP, OPS_W); });
-  mk(B, false, 0, [&](int i) { return (const double*)blk(i, T_G2); });
-  outs(T_V);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  // whitened core N and F = 2 A2 + g I
-  {
-    CombineBatch c;
-    for (int i = 0; i < MAX_BATCH; ++i) {
-      const bool ok = i < nl;
-      c.A2[i] = ok ? gops[i] + ops_block(MP, OPS_W) : nullptr;
-      c.Ac[i] = ok ? gops[i] + ops_block(MP, OPS_H) : nullptr;
-      c.V[i] = ok ? blk(i, T_V) : nullptr; c.G2[i] = ok ? blk(i, T_G2) : nullptr;
-      c.b[i] = ok ? gops[i] + ops_alpha(MP) : nullptr;
-      c.beta[i] = ok ? ops[i] + ops_beta(MP) : nullptr;
-      c.dkl[i] = ok ? gops[i] + ops_scal(MP) + SC_KL : nullptr;
-      c.clamp_flag[i] = ok ? gops[i] + ops_scal(MP) + SC_CLAMP : nullptr;
-      c.N[i] = ok ? blk(i, T_NN) : nullptr; c.F[i] = ok ? blk(i, T_F) : nullptr;
-    }
-    MOBO_LAUNCH("combine_kernel", st, combine_kernel<<<dim3((MP2 + 255) / 256, nl), 256, 0, st>>>(c, MP));
-  }
-  // dP = W^T N W
-  mk(A, false, 2, [&](int i) { return ops[i] + ops_block(MP, OPS_WT); });
-  mk(B, false, 0, [&](int i) { return (const double*)blk(i, T_NN); });
-  outs(T_X1);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  mk(A, false, 0, [&](int i) { return (const double*)blk(i, T_X1); });
-  mk(B, false, 1, [&](int i) { return ops[i] + ops_block(MP, OPS_W); });
-  outs(T_DP);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  // dLq = tril(W^T F H) - g diag(1 / Lq_ii)
-  mk(A, false, 0, [&](int i) { return (const double*)blk(i, T_F); });
-  mk(B, false, 1, [&](int i) { return ops[i] + ops_block(MP, OPS_H); });
-  outs(T_X2);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  mk(A, false, 2, [&](int i) { return ops[i] + ops_block(MP, OPS_WT); });
-  mk(B, false, 0, [&](int i) { return (const double*)blk(i, T_X2); });
-  outs(T_Y2);
-  MOBO_TRY(gemm_batched(nl, MP, A, B, C, nullptr, 1.0, 0.0, nullptr, st));
-  {
-    DlqBatch q;
-    for (int i = 0; i < MAX_BATCH; ++i) {
-      const bool ok = i < nl;
-      q.E[i] = ok ? blk(i, T_Y2) : nullptr; q.LQ[i] = ok ? ops[i] + ops_block(MP, OPS_LQ) : nullptr;
-      q.dkl[i] = ok ? gops[i] + ops_scal(MP) + SC_KL : nullptr; q.dLq[i] = ok ? dLq[i] : nullptr;
-    }
-    MOBO_LAUNCH("dlq_extract_kernel", st,
-                dlq_extract_kernel<<<dim3((M * M + 255) / 256, nl), 256, 0, st>>>(q, M, MP));
-  }
-  // dm = W^T (b + g beta)
-  {
-    VecBatch v;
-    for (int i = 0; i < MAX_BATCH; ++i) {
-      const bool ok = i < nl;
-      v.WT[i] = ok ? ops[i] + ops_block(MP, OPS_WT) : nullptr;
-      v.b[i] = ok ? gops[i] + ops_alpha(MP) : nullptr;
-      v.beta[i] = ok ? ops[i] + ops_beta(MP) : nullptr;
-      v.dkl[i] = ok ? gops[i] + ops_scal(MP) + SC_KL : nullptr;
-      v.dm[i] = ok ? dm[i] : nullptr;
-    }
-    MOBO_LAUNCH("white_vec_kernel", st, white_vec_kernel<<<dim3((M + 7) / 8, nl), 256, 0, st>>>(v, M, MP));
-  }
-  // through K(Z, Z)
-  {
-    const int nblk = (M + KZB_WARPS - 1) / KZB_WARPS;
-    KzzBwdBatch o;
-    ReduceBatch r;
-    for (int i = 0; i < MAX_BATCH; ++i) {
-      const bool ok = i < nl;
-      o.dP[i] = ok ? blk(i, T_DP) : nullptr;
-      o.part_theta[i] = ok ? work[i] + T_N * MP2 : nullptr;
-      o.dzf[i] = (ok && dzf) ? dzf[i] : nullptr;
-      r.part[i] = o.part_theta[i];
-      r.out[i] = ok ? dtheta[i] : nullptr;
-      r.n[i] = ok ? theta_size(kinds[i], d) : 0;
-    }
-    MOBO_LAUNCH("kzz_bwd_kernel", st, kzz_bwd_kernel<<<dim3(nblk, nl), KZB_WARPS * 32, 0, st>>>(b, o));
-    MOBO_LAUNCH("reduce_batch_kernel", st, reduce_batch_kernel<<<dim3(1, nl), 32, 0, st>>>(r, nblk, KZB_NTH));
-  }
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
-}
-
 int mobo_layer_precompute(int kind, int d, int M, const double* Zx, const double* zf, const double* theta,
                           const double* m, const double* Lq, double jitter, double* ops, void* stream) {
-  return mobo_model_precompute(1, &kind, d, M, &Zx, &zf, &theta, &m, &Lq, jitter, &ops, stream);
+  return model_precompute(1, &kind, d, M, &Zx, &zf, &theta, &m, &Lq, jitter, &ops, (cudaStream_t)stream, true);
 }
 
+// m and Lq reach the backward through the operators built from them (beta, H, LQ)
 int mobo_layer_precompute_bwd(int kind, int d, int M, const double* Zx, const double* zf, const double* theta,
                               const double* m, const double* Lq, const double* ops, const double* gops,
                               double* work, double* dtheta, double* dzf, double* dm, double* dLq, void* stream) {
-  return mobo_model_precompute_bwd(1, &kind, d, M, &Zx, &zf, &theta, &m, &Lq, &ops, &gops, &work, &dtheta, &dzf, &dm,
-                                   &dLq, stream);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int MP = padded(M);
+  if (d > kMaxD || MP > MAX_MP) return -2;
+  const size_t MP2 = (size_t)MP * MP;
+  // work: eight MP x MP blocks, then the per-CTA partials of kzz_bwd_kernel
+  double* G2 = work;
+  double* V = G2 + MP2;
+  double* N = V + MP2;
+  double* F = N + MP2;
+  double* X1 = F + MP2;
+  double* dP = X1 + MP2;
+  double* X2 = dP + MP2;
+  double* Y2 = X2 + MP2;
+  double* part = Y2 + MP2;
+  const double* W = ops + ops_block(MP, OPS_W);
+  const double* WT = ops + ops_block(MP, OPS_WT);
+  const double* H = ops + ops_block(MP, OPS_H);
+  const double* beta = ops + ops_beta(MP);
+  const double* A2 = gops + ops_block(MP, OPS_W);
+  const double* b = gops + ops_alpha(MP);
+  const double* dkl = gops + ops_scal(MP) + SC_KL;
+  // G2 = H H^T
+  MOBO_TRY(gemm(MP, {H, false, 1}, {H, true, 2}, G2, st));
+  // V = A2 G2
+  MOBO_TRY(gemm(MP, {A2, false, 0}, {G2, false, 0}, V, st));
+  // whitened core N and F = 2 A2 + g I
+  MOBO_LAUNCH("combine_kernel", st,
+              combine_kernel<<<(unsigned)((MP2 + 255) / 256), 256, 0, st>>>(
+                  A2, gops + ops_block(MP, OPS_H), V, G2, b, beta, dkl, gops + ops_scal(MP) + SC_CLAMP, N, F, MP));
+  // dP = W^T N W
+  MOBO_TRY(gemm(MP, {WT, false, 2}, {N, false, 0}, X1, st));
+  MOBO_TRY(gemm(MP, {X1, false, 0}, {W, false, 1}, dP, st));
+  // dLq = tril(W^T F H) - g diag(1 / Lq_ii)
+  MOBO_TRY(gemm(MP, {F, false, 0}, {H, false, 1}, X2, st));
+  MOBO_TRY(gemm(MP, {WT, false, 2}, {X2, false, 0}, Y2, st));
+  MOBO_LAUNCH("dlq_extract_kernel", st,
+              dlq_extract_kernel<<<(M * M + 255) / 256, 256, 0, st>>>(Y2, ops + ops_block(MP, OPS_LQ), dkl, dLq, M, MP));
+  // dm = W^T (b + g beta)
+  MOBO_LAUNCH("white_vec_kernel", st, white_vec_kernel<<<(M + 7) / 8, 256, 0, st>>>(WT, b, beta, dkl, dm, M, MP));
+  // through K(Z, Z)
+  const int nblk = (M + KZB_WARPS - 1) / KZB_WARPS;
+  MOBO_LAUNCH("kzz_bwd_kernel", st,
+              kzz_bwd_kernel<<<nblk, KZB_WARPS * 32, 0, st>>>(kind, d, M, MP, Zx, zf, theta, dP, part, dzf));
+  MOBO_LAUNCH("reduce_batch_kernel", st,
+              reduce_batch_kernel<<<1, 32, 0, st>>>(part, nblk, kMaxTheta, theta_size(kind, d), dtheta));
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
 static void fill_row_args(RowArgs& a, int kind, int d, int M, const double* Zx, const double* zf,
@@ -270,15 +175,24 @@ int mobo_layer_rows_fwd(int kind, int d, int M, const double* Zx, const double* 
   return launch_row_fwd(a, (cudaStream_t)stream);
 }
 
-// the whitened statistics of one layer's backward (SYRK): A2, Ac, b into the operator-gradient buffer
-static int rows_bwd_stats(int MP, long long R, int training, const double* Tsave, const double* dmu,
-                          const double* dvar, const double* craw, const unsigned int* clamp_count, double* part_syrk,
-                          double* part_alpha, double* gops, cudaStream_t st) {
-  MOBO_TRY(launch_syrk(Tsave, dvar, craw, 0, MP, R, part_syrk, gops + ops_block(MP, OPS_W), clamp_count, dmu,
-                       part_alpha, gops + ops_alpha(MP), nullptr, st));
-  MOBO_TRY(launch_syrk(Tsave, dvar, craw, 1, MP, R, part_syrk, gops + ops_block(MP, OPS_H),
-                       training ? clamp_count : nullptr, nullptr, nullptr, nullptr,
-                       gops + ops_scal(MP) + SC_CLAMP, st));
+// the whitened statistics of one layer's backward (SYRK): A2, Ac, b into the operator-gradient buffer.  One launch
+// for both weight sets (all rows -> part, clamped rows -> part_clamped; clamp_count NULL: none clamped), then the
+// fixed-order fold of the partials (latency-bound), which may run on another stream `rs` once `ev` (recorded on `st`
+// behind the SYRK) has fired
+static int rows_bwd_stats(int MP, long long R, const double* Tsave, const double* dmu, const double* dvar,
+                          const double* craw, const unsigned int* clamp_count, double* part, double* part_clamped,
+                          double* part_alpha, double* gops, cudaStream_t st, cudaStream_t rs = nullptr,
+                          cudaEvent_t ev = nullptr) {
+  MOBO_TRY(launch_syrk_both(Tsave, dvar, craw, MP, R, part, part_clamped, clamp_count, dmu, part_alpha, st));
+  cudaStream_t r = st;
+  if (rs && ev) {
+    if (cudaEventRecord(ev, st) != cudaSuccess || cudaStreamWaitEvent(rs, ev, 0) != cudaSuccess) return -1;
+    r = rs;
+  }
+  MOBO_TRY(launch_syrk_reduce(0, MP, R, part, gops + ops_block(MP, OPS_W), clamp_count, part_alpha,
+                              gops + ops_alpha(MP), nullptr, r));
+  MOBO_TRY(launch_syrk_reduce(1, MP, R, part_clamped, gops + ops_block(MP, OPS_H), clamp_count, nullptr, nullptr,
+                              gops + ops_scal(MP) + SC_CLAMP, r));
   return 0;
 }
 
@@ -291,7 +205,7 @@ static int rows_bwd_main(RowArgs& a, int kind, int d, int M, long long R, double
   const int grid = kgrad_grid(R);
   a.dk = dk;
   a.part_theta = part;
-  a.part_zf = part + (size_t)grid * MAX_THETA;
+  a.part_zf = part + (size_t)grid * kMaxTheta;
   MOBO_TRY(launch_row_bwd(a, st));
   if (a.want_param_grads && dtheta) {
     cudaStream_t r = st;
@@ -299,7 +213,7 @@ static int rows_bwd_main(RowArgs& a, int kind, int d, int M, long long R, double
       if (cudaEventRecord(ev, st) != cudaSuccess || cudaStreamWaitEvent(rs, ev, 0) != cudaSuccess) return -1;
       r = rs;
     }
-    MOBO_TRY(launch_reduce_partials(a.part_theta, grid, theta_size(kind, d), MAX_THETA, dtheta, 0, r));
+    MOBO_TRY(launch_reduce_partials(a.part_theta, grid, theta_size(kind, d), kMaxTheta, dtheta, 0, r));
     if (kind == 1 && dzf) MOBO_TRY(launch_reduce_partials(a.part_zf, grid, M, MP, dzf, 0, r));
   }
   return 0;
@@ -332,10 +246,13 @@ int mobo_layer_rows_bwd(int kind, int d, int M, const double* Zx, const double* 
   const int grid = kgrad_grid(R);
   double* dk = work;                                             // [R][MP] scratch, first so that it stays aligned
   double* part = work + mobo_rows_save_doubles(M, R);
-  double* part_syrk = part + (size_t)grid * (MAX_THETA + MP);
-  double* part_alpha = part_syrk + syrk_part_doubles(MP, R);
+  double* part_syrk = part + (size_t)grid * (kMaxTheta + MP);
+  double* part_clamped = part_syrk + syrk_part_doubles(MP, R);
+  double* part_alpha = part_clamped + syrk_part_doubles(MP, R);
   MOBO_TRY(rows_bwd_main(a, kind, d, M, R, dk, part, dtheta, dzf, st));
-  if (gops) MOBO_TRY(rows_bwd_stats(MP, R, training, Tsave, dmu, dvar, craw, clamp_count, part_syrk, part_alpha, gops, st));
+  if (gops)
+    MOBO_TRY(rows_bwd_stats(MP, R, Tsave, dmu, dvar, craw, training ? clamp_count : nullptr, part_syrk, part_clamped,
+                            part_alpha, gops, st));
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
@@ -345,14 +262,14 @@ int mobo_layer_rows_bwd(int kind, int d, int M, const double* Zx, const double* 
 namespace {
 
 struct StepLayout {
-  size_t theta[ST_MAX_LAYERS], ops[ST_MAX_LAYERS], gops[ST_MAX_LAYERS], mu[ST_MAX_LAYERS], var[ST_MAX_LAYERS],
-      craw[ST_MAX_LAYERS], dmu[ST_MAX_LAYERS], dvar[ST_MAX_LAYERS], df[ST_MAX_LAYERS], Ts[ST_MAX_LAYERS],
-      Us[ST_MAX_LAYERS], dtheta_rows[ST_MAX_LAYERS], dtheta_pre[ST_MAX_LAYERS], dzf_rows[ST_MAX_LAYERS],
-      dzf_pre[ST_MAX_LAYERS], dm_pre[ST_MAX_LAYERS], dLq_tmp[ST_MAX_LAYERS], pre_work[ST_MAX_LAYERS],
-      ell_part[ST_MAX_LAYERS], stats0[ST_MAX_LAYERS], stats1[ST_MAX_LAYERS], stats_alpha[ST_MAX_LAYERS],
-      kg_part[ST_MAX_LAYERS];
-  long long R[ST_MAX_LAYERS];
-  int ell_blocks[ST_MAX_LAYERS];
+  size_t theta[kMaxLayers], ops[kMaxLayers], gops[kMaxLayers], mu[kMaxLayers], var[kMaxLayers],
+      craw[kMaxLayers], dmu[kMaxLayers], dvar[kMaxLayers], df[kMaxLayers], Ts[kMaxLayers],
+      Us[kMaxLayers], dtheta_rows[kMaxLayers], dtheta_pre[kMaxLayers], dzf_rows[kMaxLayers],
+      dzf_pre[kMaxLayers], dm_pre[kMaxLayers], dLq_tmp[kMaxLayers], pre_work[kMaxLayers],
+      ell_part[kMaxLayers], stats0[kMaxLayers], stats1[kMaxLayers], stats_alpha[kMaxLayers],
+      kg_part[kMaxLayers];
+  long long R[kMaxLayers];
+  int ell_blocks[kMaxLayers];
   size_t noise, clamp, rows_work, total;
 };
 
@@ -361,26 +278,26 @@ StepLayout step_layout(int L, int d, int M, int S, long long B) {
   size_t off = 0;
   auto take = [&](size_t n) { const size_t o = off; off += (n + 15) / 16 * 16; return o; };
   const int MP = padded(M);
-  y.noise = take(ST_MAX_LAYERS);
-  y.clamp = take(ST_MAX_LAYERS);
+  y.noise = take(kMaxLayers);
+  y.clamp = take(kMaxLayers);
   size_t rows_work = 0;
   for (int l = 0; l < L; ++l) {
     const long long R = l == 0 ? B : B * (long long)S;
     y.R[l] = R;
     y.ell_blocks[l] = (int)((R + ELL_THREADS - 1) / ELL_THREADS);
-    y.theta[l] = take(ST_MAX_THETA);
+    y.theta[l] = take(kMaxTheta);
     y.ops[l] = take(ops_size(MP));
     y.gops[l] = take(ops_size(MP));
     y.mu[l] = take(R); y.var[l] = take(R); y.craw[l] = take(R);
     y.dmu[l] = take(R); y.dvar[l] = take(R); y.df[l] = take(R);
     y.Ts[l] = take(mobo_rows_save_doubles(M, R));
     y.Us[l] = take(mobo_rows_save_doubles(M, R));
-    y.dtheta_rows[l] = take(ST_MAX_THETA); y.dtheta_pre[l] = take(ST_MAX_THETA);
+    y.dtheta_rows[l] = take(kMaxTheta); y.dtheta_pre[l] = take(kMaxTheta);
     y.dzf_rows[l] = take(MP); y.dzf_pre[l] = take(MP); y.dm_pre[l] = take(MP);
     y.dLq_tmp[l] = take((size_t)M * M);
     y.pre_work[l] = take(mobo_precompute_bwd_work_doubles(M));
     y.ell_part[l] = take(2 * (size_t)y.ell_blocks[l]);
-    const size_t w = mobo_rows_save_doubles(M, R) + (size_t)256 * KG_CTAS_PER_SM * (MAX_THETA + MP) + 64;
+    const size_t w = mobo_rows_save_doubles(M, R) + (size_t)256 * KG_CTAS_PER_SM * (kMaxTheta + MP) + 64;
     rows_work = w > rows_work ? w : rows_work;
     // SYRK partials per layer and per weight set: their fold runs on the side stream while the main stream is already
     // in the next layer's SYRK
@@ -388,7 +305,7 @@ StepLayout step_layout(int L, int d, int M, int S, long long B) {
     y.stats1[l] = take(syrk_part_doubles(MP, R));
     y.stats_alpha[l] = take(syrk_alpha_doubles(MP, syrk_nchunk(MP, R)) + 64);
     // per-CTA partials of the covariance-gradient kernel, per layer: their fold runs on the side stream too
-    y.kg_part[l] = take((size_t)256 * KG_CTAS_PER_SM * (MAX_THETA + MP) + 64);
+    y.kg_part[l] = take((size_t)256 * KG_CTAS_PER_SM * (kMaxTheta + MP) + 64);
   }
   y.rows_work = take(rows_work);
   y.total = off;
@@ -406,14 +323,14 @@ StepLayout step_layout(int L, int d, int M, int S, long long B) {
 // lock on first use - the only state this library keeps.
 namespace {
 struct SideCtx {
-  int device = -1; cudaStream_t s = nullptr; cudaEvent_t fork[ST_MAX_LAYERS]; cudaEvent_t join = nullptr;
-  cudaEvent_t done[ST_MAX_LAYERS];      // layer l's operator-chain backward (its d L_q, d m, d theta shares) is complete
-  cudaEvent_t kg[ST_MAX_LAYERS];        // layer l's covariance-gradient kernel is complete (its partials may be folded)
+  int device = -1; cudaStream_t s = nullptr; cudaEvent_t fork[kMaxLayers]; cudaEvent_t join = nullptr;
+  cudaEvent_t done[kMaxLayers];      // layer l's operator-chain backward (its d L_q, d m, d theta shares) is complete
+  cudaEvent_t kg[kMaxLayers];        // layer l's covariance-gradient kernel is complete (its partials may be folded)
 };
 bool side_ctx_init(SideCtx& c) {
   if (cudaGetDevice(&c.device) != cudaSuccess) return false;
   if (cudaStreamCreateWithFlags(&c.s, cudaStreamNonBlocking) != cudaSuccess) return false;
-  for (int i = 0; i < ST_MAX_LAYERS; ++i)
+  for (int i = 0; i < kMaxLayers; ++i)
     if (cudaEventCreateWithFlags(&c.fork[i], cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&c.done[i], cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&c.kg[i], cudaEventDisableTiming) != cudaSuccess) return false;
@@ -438,14 +355,14 @@ void* mobo_step_ctx_create(void) {
 }
 int mobo_step_ctx_wait_layer(void* ctx, int layer, void* stream) {
   SideCtx* c = static_cast<SideCtx*>(ctx);
-  if (!c || layer < 0 || layer >= ST_MAX_LAYERS) return -2;
+  if (!c || layer < 0 || layer >= kMaxLayers) return -2;
   return cudaStreamWaitEvent((cudaStream_t)stream, c->done[layer], 0) == cudaSuccess ? 0 : -1;
 }
 void mobo_step_ctx_destroy(void* ctx) {
   SideCtx* c = static_cast<SideCtx*>(ctx);
   if (!c) return;
   if (c->s) cudaStreamDestroy(c->s);
-  for (int i = 0; i < ST_MAX_LAYERS; ++i) { if (c->fork[i]) cudaEventDestroy(c->fork[i]); if (c->done[i]) cudaEventDestroy(c->done[i]); if (c->kg[i]) cudaEventDestroy(c->kg[i]); }
+  for (int i = 0; i < kMaxLayers; ++i) { if (c->fork[i]) cudaEventDestroy(c->fork[i]); if (c->done[i]) cudaEventDestroy(c->done[i]); if (c->kg[i]) cudaEventDestroy(c->kg[i]); }
   if (c->join) cudaEventDestroy(c->join);
   delete c;
 }
@@ -462,43 +379,39 @@ static int side_stream_sms() {      // development override: MOBO_SIDE_SMS=n
 void mobo_step_side_stream(int on) { g_side_stream_on = on != 0; }
 
 size_t mobo_elbo_step_workspace_doubles(int L, int d, int M, int S, long long B) {
-  if (L < 1 || L > ST_MAX_LAYERS) return 0;
+  if (L < 1 || L > kMaxLayers) return 0;
   return step_layout(L, d, M, S, B).total;
 }
 
 int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const int L = D->L, d = D->d, M = D->M, S = D->S < 1 ? 1 : D->S;
-  if (L < 1 || L > ST_MAX_LAYERS || d > kMaxD || padded(M) > MAX_MP || D->B < 1) return -2;
+  if (L < 1 || L > kMaxLayers || d > kMaxD || padded(M) > MAX_MP || D->B < 1) return -2;
   const int MP = padded(M);
   const StepLayout y = step_layout(L, d, M, S, D->B);
   double* ws = D->workspace;
   const double kl_scale = (double)D->B / (double)D->num_data;
   unsigned int* clamp = reinterpret_cast<unsigned int*>(ws + y.clamp);
 
-  int kinds[ST_MAX_LAYERS];
-  const double* Zx[ST_MAX_LAYERS]; const double* zf[ST_MAX_LAYERS]; const double* theta[ST_MAX_LAYERS];
-  const double* m[ST_MAX_LAYERS]; const double* Lq[ST_MAX_LAYERS];
-  double* ops[ST_MAX_LAYERS]; const double* cops[ST_MAX_LAYERS]; const double* gops[ST_MAX_LAYERS];
-  double* pre_work[ST_MAX_LAYERS]; double* dtheta_pre[ST_MAX_LAYERS]; double* dzf_pre[ST_MAX_LAYERS];
-  double* dm_pre[ST_MAX_LAYERS]; double* dLq[ST_MAX_LAYERS];
+  int kinds[kMaxLayers];
+  const double* Zx[kMaxLayers]; const double* zf[kMaxLayers]; const double* theta[kMaxLayers];
+  const double* m[kMaxLayers]; const double* Lq[kMaxLayers];
+  double* ops[kMaxLayers]; double* dLq[kMaxLayers];
   for (int l = 0; l < L; ++l) {
     const mobo_layer_desc& ld = D->layer[l];
     kinds[l] = l == 0 ? 0 : 1;
     Zx[l] = ld.Zx; zf[l] = l == 0 ? nullptr : D->layer[l - 1].m; theta[l] = ws + y.theta[l];
     m[l] = ld.m; Lq[l] = ld.Lq;
-    ops[l] = ws + y.ops[l]; cops[l] = ops[l]; gops[l] = ws + y.gops[l];
-    pre_work[l] = ws + y.pre_work[l]; dtheta_pre[l] = ws + y.dtheta_pre[l]; dzf_pre[l] = ws + y.dzf_pre[l];
-    dm_pre[l] = ws + y.dm_pre[l];
+    ops[l] = ws + y.ops[l];
     dLq[l] = (ld.g_Lq && !D->accumulate) ? ld.g_Lq : ws + y.dLq_tmp[l];
   }
   // 1. raw -> constrained
   {
     PrepArgs a;
     a.L = L; a.d = d; a.noise = ws + y.noise; a.clamp_count = clamp; a.dkl = kl_scale;
-    for (int l = 0; l < ST_MAX_LAYERS; ++l) {
+    for (int l = 0; l < kMaxLayers; ++l) {
       const bool ok = l < L;
-      for (int i = 0; i < ST_MAX_THETA; ++i) a.raw_theta[l][i] = ok ? D->layer[l].raw_theta[i] : nullptr;
+      for (int i = 0; i < kMaxTheta; ++i) a.raw_theta[l][i] = ok ? D->layer[l].raw_theta[i] : nullptr;
       a.raw_noise[l] = ok ? D->layer[l].raw_noise : nullptr;
       a.noise_lo[l] = ok ? D->layer[l].noise_lower : 0.0; a.noise_hi[l] = ok ? D->layer[l].noise_upper : 0.0;
       a.theta[l] = ok ? ws + y.theta[l] : nullptr;
@@ -509,7 +422,7 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
     MOBO_LAUNCH("step_prep_kernel", st, step_prep_kernel<<<L, 96, 0, st>>>(a));
   }
   // 2. operator chain of every layer
-  MOBO_TRY(model_precompute(L, kinds, d, M, Zx, zf, theta, m, Lq, D->jitter, ops, stream, false));
+  MOBO_TRY(model_precompute(L, kinds, d, M, Zx, zf, theta, m, Lq, D->jitter, ops, st, false));
   // 3. forward row passes, low -> high fidelity
   for (int l = 0; l < L; ++l) {
     const long long R = y.R[l];
@@ -541,16 +454,12 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
     // slower); the fold of its partials and the latency-bound operator-chain backward of this layer go to the side
     // stream
     double* gl = ws + y.gops[l];
-    MOBO_TRY(launch_syrk_both(ws + y.Ts[l], ws + y.dvar[l], ws + y.craw[l], MP, R, ws + y.stats0[l], ws + y.stats1[l],
-                              clamp + l, ws + y.dmu[l], ws + y.stats_alpha[l], st));
-    if (fork && (cudaEventRecord(sc.fork[l], st) != cudaSuccess || cudaStreamWaitEvent(ss, sc.fork[l], 0) != cudaSuccess))
-      return -1;
-    MOBO_TRY(launch_syrk_reduce(0, MP, R, ws + y.stats0[l], gl + ops_block(MP, OPS_W), clamp + l, ws + y.stats_alpha[l],
-                                gl + ops_alpha(MP), nullptr, ss));
-    MOBO_TRY(launch_syrk_reduce(1, MP, R, ws + y.stats1[l], gl + ops_block(MP, OPS_H), clamp + l, nullptr, nullptr,
-                                gl + ops_scal(MP) + SC_CLAMP, ss));
-    MOBO_TRY(mobo_model_precompute_bwd(1, kinds + l, d, M, Zx + l, zf + l, theta + l, m + l, Lq + l, cops + l, gops + l,
-                                       pre_work + l, dtheta_pre + l, dzf_pre + l, dm_pre + l, dLq + l, (void*)ss));
+    MOBO_TRY(rows_bwd_stats(MP, R, ws + y.Ts[l], ws + y.dmu[l], ws + y.dvar[l], ws + y.craw[l], clamp + l,
+                            ws + y.stats0[l], ws + y.stats1[l], ws + y.stats_alpha[l], gl, st, fork ? ss : nullptr,
+                            fork ? sc.fork[l] : nullptr));
+    MOBO_TRY(mobo_layer_precompute_bwd(kinds[l], d, M, Zx[l], zf[l], theta[l], m[l], Lq[l], ops[l], gl,
+                                       ws + y.pre_work[l], ws + y.dtheta_pre[l], ws + y.dzf_pre[l], ws + y.dm_pre[l],
+                                       dLq[l], (void*)ss));
     // d L_q of this layer is final (it is written straight into the caller's gradient): a multi-GPU caller may start
     // its all-reduce now, behind the lower layers' row kernels (mobo_step_ctx_wait_layer)
     if (scp && !D->accumulate && cudaEventRecord(sc.done[l], ss) != cudaSuccess) return -1;
@@ -572,9 +481,9 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
   {
     FinishArgs a;
     a.L = L; a.d = d; a.M = M; a.MP = MP; a.kl_scale = kl_scale; a.out = D->out; a.accumulate = D->accumulate;
-    for (int l = 0; l < ST_MAX_LAYERS; ++l) {
+    for (int l = 0; l < kMaxLayers; ++l) {
       const bool ok = l < L;
-      for (int i = 0; i < ST_MAX_THETA; ++i) {
+      for (int i = 0; i < kMaxTheta; ++i) {
         a.raw_theta[l][i] = ok ? D->layer[l].raw_theta[i] : nullptr;
         a.g_raw_theta[l][i] = ok ? D->layer[l].g_raw_theta[i] : nullptr;
       }
@@ -636,7 +545,7 @@ int mobo_acq_moments(int fidelity, int d, int M, int S, long long n, const doubl
                      const double* raw_noise, double noise_lower, double noise_upper, const double* X,
                      double* out_mu, double* out_var, double* scratch, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  if (fidelity < 0 || fidelity >= ST_MAX_LAYERS || n < 1 || S < 1) return -2;
+  if (fidelity < 0 || fidelity >= kMaxLayers || n < 1 || S < 1) return -2;
   const long long RS = n * (long long)S;
   double* mu[2] = {scratch, scratch + 2 * RS};
   double* var[2] = {scratch + RS, scratch + 3 * RS};

@@ -38,6 +38,8 @@ inline void prof_end(cudaStream_t st) {
 #define MOBO_LAUNCH(name, st, ...) do { mobo::prof_begin(name, st); __VA_ARGS__; mobo::prof_end(st); } while (0)
 
 constexpr int kMaxD = 8;               // max number of x columns (ARD dims) handled by the kernels
+constexpr int kMaxLayers = 8;          // max number of layers of a model (MOBO_MAX_LAYERS in the C header)
+constexpr int kMaxTheta = 5 + 2 * kMaxD;   // hyper-parameter slots of a layer (theta_size(1, kMaxD); MOBO_MAX_THETA)
 constexpr double kMinVariance = 1e-10; // gpytorch settings.min_variance (fp64), quirk Q9
 
 // ---- operator buffer layout (doubles), one per (model, layer); MP = M rounded up to a multiple of 32 ----
@@ -61,7 +63,7 @@ __host__ __device__ inline size_t frag_offset(int MP, int i, int k) {
 // scal[SC_CLAMP] is meaningful in the GRADIENT buffer: number of clamped rows behind block OPS_H (0 -> Ac == 0)
 // scal[SC_RETRIES]: number of psd_safe_cholesky retries the operator chain needed (0 .. 3); SC_STATUS = 1: all failed
 enum OpsScal { SC_KL = 0, SC_LOGDET_P = 1, SC_LOGDET_Q = 2, SC_BETA2 = 3, SC_H2 = 4, SC_STATUS = 5, SC_CLAMP = 6,
-               SC_RETRIES = 7, SC_COUNTER = 8 };
+               SC_RETRIES = 7 };
 __host__ __device__ inline size_t ops_block(int MP, int b) { return (size_t)b * MP * MP; }
 __host__ __device__ inline size_t ops_beta(int MP) { return (size_t)OPS_NBLOCKS * MP * MP; }
 __host__ __device__ inline size_t ops_alpha(int MP) { return (size_t)OPS_NBLOCKS * MP * MP + MP; }

@@ -1,4 +1,4 @@
-// Per-step M x M operator chain of the sparse-GP layers (forward and backward) for sm_100a, batched over layers.
+// Per-step M x M operator chain of the sparse-GP layers (forward and backward) for sm_100a.
 //
 // Forward (what the reference reaches through UnwhitenedVariationalStrategy.forward / kl_mvn_mvn [upstream gpytorch],
 // called from mobocmf/layers/mfdgp_hidden_layer.py:286 and mobocmf/mlls/variational_elbo_mf.py:40):
@@ -14,90 +14,34 @@
 // the gradient through the inducing inputs [Z, m_{l-1}] (SURVEY.md §7).
 //
 // All matrices are MP x MP row-major (MP = M rounded up to 32, identity/zero padded) and L2-resident; products run
-// on the DMMA pipe.  The layers of a model are independent here and are batched in the grid.
+// on the DMMA pipe.  The layers' chains are independent: the forward of all layers of a model is one launch
+// (opchain.cu, LayerBatch); the backward below is enqueued one layer at a time.
 #include "common.cuh"
 
 namespace mobo {
 
-constexpr int MAX_BATCH = 8;
-
 struct LayerBatch {
   int n;
   int d, M, MP;
-  int kind[MAX_BATCH];
-  const double* Zx[MAX_BATCH];
-  const double* zf[MAX_BATCH];
-  const double* theta[MAX_BATCH];
-  const double* m[MAX_BATCH];
-  const double* Lq[MAX_BATCH];
-  double* ops[MAX_BATCH];
+  int kind[kMaxLayers];
+  const double* Zx[kMaxLayers];
+  const double* zf[kMaxLayers];
+  const double* theta[kMaxLayers];
+  const double* m[kMaxLayers];
+  const double* Lq[kMaxLayers];
+  double* ops[kMaxLayers];
 };
-
-struct PtrBatch3 {
-  const double* A[MAX_BATCH];
-  const double* B[MAX_BATCH];
-  double* C[MAX_BATCH];
-  double* Ct[MAX_BATCH];   // optional transposed copy of C
-};
-
-// ---------------------------------------------------------------------------------------------------
-// covariance function between inducing inputs
-// ---------------------------------------------------------------------------------------------------
-__global__ void kzz_kernel(LayerBatch b, double jitter, int block_index /* which ops block receives P */,
-                           int reset_counter /* zero finalize_kernel's arrival counter: ops is caller memory */) {
-  __shared__ KernParams kp;
-  const int bi = blockIdx.y;
-  const int kind = b.kind[bi], d = b.d, M = b.M, MP = b.MP;
-  if (reset_counter && blockIdx.x == 0 && threadIdx.x == 0)
-    *reinterpret_cast<unsigned long long*>(b.ops[bi] + ops_scal(MP) + SC_COUNTER) = 0ull;
-  const double* Zx = b.Zx[bi];
-  const double* zf = b.zf[bi];
-  if (threadIdx.x == 0) load_kern_params(kp, kind, d, b.theta[bi]);
-  __syncthreads();
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= MP * MP) return;
-  const int i = idx / MP, j = idx - i * MP;
-  double val;
-  if (i >= M || j >= M) {
-    val = (i == j) ? 1.0 : 0.0;
-  } else if (i == j) {
-    val = kern_diag(kp, kind == 1 ? zf[i] : 0.0) + jitter;
-  } else {
-    double D1 = 0.0, D2 = 0.0;
-    for (int c = 0; c < d; ++c) {
-      const double df = Zx[(size_t)i * d + c] - Zx[(size_t)j * d + c];
-      D1 = fma(df * df, kp.il1[c], D1);
-      D2 = fma(df * df, kp.il2[c], D2);
-    }
-    const double E1 = exp(-0.5 * D1);
-    if (kind == 0) {
-      val = kp.a1 * E1;
-    } else {
-      const double fi = zf[i], fj = zf[j], dff = fi - fj;
-      val = kp.a1 * E1 * (kp.vlin * fi * fj + kp.af * exp(-0.5 * dff * dff * kp.ilf)) + kp.a2 * exp(-0.5 * D2);
-    }
-  }
-  (b.ops[bi] + ops_block(MP, block_index))[idx] = val;
-}
 
 // backward through K(Z,Z): dP symmetric.  One warp per inducing point i.
 //   dtheta += sum_ij dP_ij dk_ij/dtheta ;  dzf_i = 2 sum_j dP_ij dk(z_i,z_j)/d f_i
+//   part_theta: [gridDim.x][kMaxTheta];  dzf: M or NULL
 constexpr int KZB_WARPS = 8;
-constexpr int KZB_NTH = 5 + 2 * kMaxD;
-struct KzzBwdBatch {
-  const double* dP[MAX_BATCH];
-  double* part_theta[MAX_BATCH];   // [gridDim.x][KZB_NTH]
-  double* dzf[MAX_BATCH];
-};
-__global__ void __launch_bounds__(KZB_WARPS * 32) kzz_bwd_kernel(LayerBatch b, KzzBwdBatch o) {
+__global__ void __launch_bounds__(KZB_WARPS * 32)
+kzz_bwd_kernel(int kind, int d, int M, int MP, const double* Zx, const double* zf, const double* theta,
+               const double* dP, double* part_theta, double* dzf) {
   __shared__ KernParams kp;
-  __shared__ double accw[KZB_WARPS][KZB_NTH];
-  const int bi = blockIdx.y;
-  const int kind = b.kind[bi], d = b.d, M = b.M, MP = b.MP;
-  const double* Zx = b.Zx[bi];
-  const double* zf = b.zf[bi];
-  const double* dP = o.dP[bi];
-  if (threadIdx.x == 0) load_kern_params(kp, kind, d, b.theta[bi]);
+  __shared__ double accw[KZB_WARPS][kMaxTheta];
+  if (threadIdx.x == 0) load_kern_params(kp, kind, d, theta);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int i = blockIdx.x * KZB_WARPS + warp;
@@ -162,7 +106,7 @@ __global__ void __launch_bounds__(KZB_WARPS * 32) kzz_bwd_kernel(LayerBatch b, K
     }
   }
   dzi = warp_sum(dzi);
-  if (lane == 0 && i < M && kind == 1 && o.dzf[bi]) o.dzf[bi][i] = 2.0 * dzi;
+  if (lane == 0 && i < M && kind == 1 && dzf) dzf[i] = 2.0 * dzi;
 #pragma unroll
   for (int q = 0; q < 5; ++q) {
     const double s = warp_sum(th_s[q]);
@@ -177,7 +121,7 @@ __global__ void __launch_bounds__(KZB_WARPS * 32) kzz_bwd_kernel(LayerBatch b, K
   }
   __syncthreads();
   const int tid = threadIdx.x;
-  if (tid < KZB_NTH) {
+  if (tid < kMaxTheta) {
     double s = 0.0;
     for (int w = 0; w < KZB_WARPS; ++w) s += accw[w][tid];
     double out = 0.0;
@@ -194,19 +138,17 @@ __global__ void __launch_bounds__(KZB_WARPS * 32) kzz_bwd_kernel(LayerBatch b, K
         out = s * kp.il2[c] * sqrt(kp.il2[c]);
       }
     }
-    if (slot >= 0) o.part_theta[bi][(size_t)blockIdx.x * KZB_NTH + slot] = out;
+    if (slot >= 0) part_theta[(size_t)blockIdx.x * kMaxTheta + slot] = out;
   }
 }
 
-// out[bi][i] = sum_b part[bi][b][i]  (fixed order)
-struct ReduceBatch { const double* part[MAX_BATCH]; double* out[MAX_BATCH]; int n[MAX_BATCH]; };
-__global__ void reduce_batch_kernel(ReduceBatch r, int nblocks, int stride) {
-  const int bi = blockIdx.y;
+// out[i] = sum_b part[b][i], i < n  (sequential in b: a fixed order)
+__global__ void reduce_batch_kernel(const double* part, int nblocks, int stride, int n, double* out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= r.n[bi]) return;
+  if (i >= n) return;
   double s = 0.0;
-  for (int b = 0; b < nblocks; ++b) s += r.part[bi][(size_t)b * stride + i];
-  r.out[bi][i] = s;
+  for (int b = 0; b < nblocks; ++b) s += part[(size_t)b * stride + i];
+  out[i] = s;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -234,7 +176,7 @@ __device__ __forceinline__ void chol32_inwarp(double (&row)[32], double& rinv, i
 }
 
 // ---------------------------------------------------------------------------------------------------
-// batched strided GEMM  C = alpha op(A) op(B) + beta C  (n x n x n, n multiple of 32), 32x32 tiles, BK = 32,
+// strided GEMM  C = op(A) op(B)  (n x n x n, n multiple of 32), 32x32 tiles, BK = 32,
 // register-prefetched double buffering.  Triangular operands shorten the k range:
 //   a_tri: 1 = op(A)[m][k] == 0 for k > m (lower), 2 = == 0 for k < m (upper);  b_tri likewise on op(B)[k][n]:
 //   1 = lower (== 0 for n > k), 2 = upper (== 0 for n < k).
@@ -246,20 +188,17 @@ struct GemmArgs {
   int n;
   int rsA, csA, rsB, csB;
   int a_tri, b_tri;
-  double alpha, beta;
-  const double* skip_if_zero[MAX_BATCH];   // optional per-entry device flag: skip the entry when *flag == 0
-  PtrBatch3 p;
+  const double* A;
+  const double* B;
+  double* C;
 };
 
 __global__ void __launch_bounds__(GM_THREADS) gemm_kernel(const __grid_constant__ GemmArgs a) {
-  if (a.skip_if_zero[blockIdx.z] && *a.skip_if_zero[blockIdx.z] == 0.0) return;
   __shared__ double As[2][GM_K][GM_LD];   // [k][m]
   __shared__ double Bs[2][GM_K][GM_LD];   // [k][n]
-  const int bi = blockIdx.z;
-  const double* __restrict__ A = a.p.A[bi];
-  const double* __restrict__ B = a.p.B[bi];
-  double* __restrict__ C = a.p.C[bi];
-  double* __restrict__ Ct = a.p.Ct[bi];
+  const double* __restrict__ A = a.A;
+  const double* __restrict__ B = a.B;
+  double* __restrict__ C = a.C;
   const int n = a.n;
   const int m0 = blockIdx.y * GM_T, n0 = blockIdx.x * GM_T;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -327,88 +266,66 @@ __global__ void __launch_bounds__(GM_THREADS) gemm_kernel(const __grid_constant_
 #pragma unroll
       for (int e = 0; e < 2; ++e) {
         const int i = m0 + 16 * wi + 8 * x + g, j = n0 + 16 * wj + 8 * y + 2 * t + e;
-        const size_t o = (size_t)i * n + j;
-        const double v = a.alpha * acc[x][y][e] + (a.beta != 0.0 ? a.beta * C[o] : 0.0);
-        C[o] = v;
-        if (Ct) Ct[(size_t)j * n + i] = v;
+        C[(size_t)i * n + j] = acc[x][y][e];
       }
 }
 
-struct GemmOperand { const double* p[MAX_BATCH]; bool trans; int tri; };
+// an operand of gemm(): op(p) = p^T when trans; tri as a_tri / b_tri above
+struct GemmOperand { const double* p; bool trans; int tri; };
 
-static int gemm_batched(int nbatch, int n, const GemmOperand& A, const GemmOperand& B, double* const* C,
-                        double* const* Ct, double alpha, double beta, const double* const* skip_if_zero,
-                        cudaStream_t st) {
+static int gemm(int n, const GemmOperand& A, const GemmOperand& B, double* C, cudaStream_t st) {
   GemmArgs a;
   a.n = n;
   a.rsA = A.trans ? 1 : n; a.csA = A.trans ? n : 1;
   a.rsB = B.trans ? 1 : n; a.csB = B.trans ? n : 1;
   a.a_tri = A.tri; a.b_tri = B.tri;
-  a.alpha = alpha; a.beta = beta;
-  for (int i = 0; i < MAX_BATCH; ++i) {
-    a.p.A[i] = i < nbatch ? A.p[i] : nullptr;
-    a.p.B[i] = i < nbatch ? B.p[i] : nullptr;
-    a.p.C[i] = i < nbatch ? C[i] : nullptr;
-    a.p.Ct[i] = (i < nbatch && Ct) ? Ct[i] : nullptr;
-    a.skip_if_zero[i] = (i < nbatch && skip_if_zero) ? skip_if_zero[i] : nullptr;
-  }
-  dim3 grid(n / GM_T, n / GM_T, nbatch);
-  MOBO_LAUNCH("gemm_kernel", st, gemm_kernel<<<grid, GM_THREADS, 0, st>>>(a));
+  a.A = A.p; a.B = B.p; a.C = C;
+  MOBO_LAUNCH("gemm_kernel", st, gemm_kernel<<<dim3(n / GM_T, n / GM_T), GM_THREADS, 0, st>>>(a));
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
 // dm = W^T (b + g beta).  Warp per row of W^T.
-struct VecBatch {
-  const double* WT[MAX_BATCH]; const double* b[MAX_BATCH]; const double* beta[MAX_BATCH]; const double* dkl[MAX_BATCH];
-  double* dm[MAX_BATCH];
-};
-__global__ void __launch_bounds__(256) white_vec_kernel(VecBatch v, int M, int MP) {
-  const int bi = blockIdx.y;
+__global__ void __launch_bounds__(256) white_vec_kernel(const double* WT, const double* b, const double* beta,
+                                                        const double* dkl, double* dm, int M, int MP) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int j = blockIdx.x * 8 + warp;
   if (j >= M) return;
-  const double* row = v.WT[bi] + (size_t)j * MP;
-  const double g = v.dkl[bi][0];
+  const double* row = WT + (size_t)j * MP;
+  const double g = dkl[0];
   double s = 0.0;
-  for (int i = j + lane; i < MP; i += 32) s = fma(row[i], v.b[bi][i] + g * v.beta[bi][i], s);
+  for (int i = j + lane; i < MP; i += 32) s = fma(row[i], b[i] + g * beta[i], s);
   s = warp_sum(s);
-  if (lane == 0) v.dm[bi][j] = s;
+  if (lane == 0) dm[j] = s;
 }
 
 // whitened gradient core  N = A1 - V - V^T - 1/2 (beta b^T + b beta^T) + g/2 (I - beta beta^T - G2)  (dP = W^T N W)
 // and F = 2 A2 + g I  (dLq = tril(W^T F H) - g diag(1/Lq_ii));  A1 = A2 - Ac when some row was clamped.
-struct CombineBatch {
-  const double* A2[MAX_BATCH]; const double* Ac[MAX_BATCH]; const double* V[MAX_BATCH]; const double* G2[MAX_BATCH];
-  const double* b[MAX_BATCH]; const double* beta[MAX_BATCH]; const double* dkl[MAX_BATCH];
-  const double* clamp_flag[MAX_BATCH]; double* N[MAX_BATCH]; double* F[MAX_BATCH];
-};
-__global__ void combine_kernel(CombineBatch c, int MP) {
-  const int bi = blockIdx.y;
+//   clamp_flag: number of clamped rows (scal[SC_CLAMP] of the gradient buffer)
+__global__ void combine_kernel(const double* A2, const double* Ac, const double* V, const double* G2, const double* b,
+                               const double* beta, const double* dkl, const double* clamp_flag, double* N, double* F,
+                               int MP) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= MP * MP) return;
   const int i = idx / MP, j = idx - i * MP;
   const size_t tr = (size_t)j * MP + i;
-  const double g = c.dkl[bi][0];
-  const bool clamped = c.clamp_flag[bi] && *c.clamp_flag[bi] != 0.0;
-  const double a2 = 0.5 * (c.A2[bi][idx] + c.A2[bi][tr]);
-  const double a1 = clamped ? a2 - 0.5 * (c.Ac[bi][idx] + c.Ac[bi][tr]) : a2;
-  const double bi_ = c.b[bi][i], bj_ = c.b[bi][j], be_i = c.beta[bi][i], be_j = c.beta[bi][j];
+  const double g = dkl[0];
+  const bool clamped = *clamp_flag != 0.0;
+  const double a2 = 0.5 * (A2[idx] + A2[tr]);
+  const double a1 = clamped ? a2 - 0.5 * (Ac[idx] + Ac[tr]) : a2;
+  const double bi_ = b[i], bj_ = b[j], be_i = beta[i], be_j = beta[j];
   const double eye = i == j ? 1.0 : 0.0;
-  c.N[bi][idx] = a1 - c.V[bi][idx] - c.V[bi][tr] - 0.5 * (be_i * bj_ + bi_ * be_j) +
-                 0.5 * g * (eye - be_i * be_j - c.G2[bi][idx]);
-  c.F[bi][idx] = 2.0 * a2 + g * eye;
+  N[idx] = a1 - V[idx] - V[tr] - 0.5 * (be_i * bj_ + bi_ * be_j) + 0.5 * g * (eye - be_i * be_j - G2[idx]);
+  F[idx] = 2.0 * a2 + g * eye;
 }
 
 // dLq (M x M, ld M) = tril(E)[:M,:M] - g diag(1 / Lq_ii)
-struct DlqBatch { const double* E[MAX_BATCH]; const double* LQ[MAX_BATCH]; const double* dkl[MAX_BATCH]; double* dLq[MAX_BATCH]; };
-__global__ void dlq_extract_kernel(DlqBatch q, int M, int MP) {
-  const int bi = blockIdx.y;
+__global__ void dlq_extract_kernel(const double* E, const double* LQ, const double* dkl, double* dLq, int M, int MP) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= M * M) return;
   const int i = idx / M, j = idx - i * M;
-  double v = j <= i ? q.E[bi][(size_t)i * MP + j] : 0.0;
-  if (i == j) v -= q.dkl[bi][0] / q.LQ[bi][(size_t)i * MP + i];
-  q.dLq[bi][idx] = v;
+  double v = j <= i ? E[(size_t)i * MP + j] : 0.0;
+  if (i == j) v -= dkl[0] / LQ[(size_t)i * MP + i];
+  dLq[idx] = v;
 }
 
 }  // namespace mobo

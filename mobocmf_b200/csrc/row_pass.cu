@@ -46,7 +46,6 @@ constexpr int NHALF = TR / 32;     // 32-column groups of the tile; warps = NHAL
 constexpr int ROW_CTAS_PER_SM = 2; // two CTAs per SM fill each other's phase boundaries (K build <-> DMMA products)
 constexpr int MAX_MP = 256;        // slab scheme: (MP/32) warp pairs <= 8
 constexpr int NCH_MAX = MAX_MP / 32;
-constexpr int MAX_THETA = 5 + 2 * kMaxD;
 
 struct RowArgs {
   int kind, d, M, MP;
@@ -77,7 +76,7 @@ struct RowArgs {
   double* dk;              // scratch [R][MP]: d loss / d K(z_j, row r), written by the product kernel, read by kgrad
   double* df;              // R: d loss / d f_r   (kind 1)
   double* dxrow;           // optional R x d: d loss / d x of each row
-  double* part_theta;      // [grid][MAX_THETA]
+  double* part_theta;      // [grid][kMaxTheta]
   double* part_zf;         // [grid][MP]
   int want_param_grads;
   int want_x_grads;
@@ -140,7 +139,7 @@ struct CovSmem {
   double zsT[kMaxD][MAX_MP];
   double zfs[MAX_MP];
   double acc_zf[BWD ? NW : 1][BWD ? MAX_MP : 1];   // backward: per-warp d zf accumulators
-  double acc_th[BWD ? NW : 1][MAX_THETA];   // backward: per-warp d theta accumulators (scalars | l1 | l2)
+  double acc_th[BWD ? NW : 1][kMaxTheta];   // backward: per-warp d theta accumulators (scalars | l1 | l2)
 };
 
 struct RowSmem : CovSmem<ROW_WARPS, false> {
@@ -1470,7 +1469,7 @@ __global__ void __launch_bounds__(KG_THREADS, KG_CTAS_PER_SM) kgrad_kernel(const
 
   load_inducing(a, sm);
   for (int j = lane; j < MAX_MP; j += 32) sm.acc_zf[warp][j] = 0.0;
-  if (lane < MAX_THETA) sm.acc_th[warp][lane] = 0.0;
+  if (lane < kMaxTheta) sm.acc_th[warp][lane] = 0.0;
   __syncthreads();
 
   // every warp walks its own groups of RPW rows: the rows' state lives in the warp's slice of the shared arrays and
@@ -1520,7 +1519,7 @@ __global__ void __launch_bounds__(KG_THREADS, KG_CTAS_PER_SM) kgrad_kernel(const
       for (int w = 0; w < KG_WARPS; ++w) s += sm.acc_zf[w][j];
       a.part_zf[(size_t)blockIdx.x * MP + j] = s;
     }
-    if (tid < MAX_THETA) {
+    if (tid < kMaxTheta) {
       double s = 0.0;
       for (int w = 0; w < KG_WARPS; ++w) s += sm.acc_th[w][tid];
       // map (scalars | l1 | l2) accumulators to the theta layout and undo the accumulator scalings (see kgrad_tile)
@@ -1546,7 +1545,7 @@ __global__ void __launch_bounds__(KG_THREADS, KG_CTAS_PER_SM) kgrad_kernel(const
           out = s * kf.il2[c] * sqrt(kf.il2[c]);
         }
       }
-      if (slot >= 0) a.part_theta[(size_t)blockIdx.x * MAX_THETA + slot] = out;
+      if (slot >= 0) a.part_theta[(size_t)blockIdx.x * kMaxTheta + slot] = out;
     }
   }
 }
@@ -1572,8 +1571,9 @@ __global__ void reduce_partials_kernel(const double* __restrict__ part, int nblo
 // twelve consumer warps have released it (one "empty" mbarrier per slot), so the consumers drift up to two stages
 // apart instead of meeting at a CTA barrier every 8 k-steps.
 // Partial blocks per row chunk are folded in chunk order by syrk_reduce_kernel, which also mirrors the result to
-// the full symmetric matrix.  w_r = dvar_r (which = 0) or dvar_r * [clamped row] (which = 1, skipped unless some
-// row was clamped).  Group 0 also accumulates b = sum_r dmu_r t_r.
+// the full symmetric matrix.  One launch computes both weight sets, which = blockIdx.z: w_r = dvar_r (which = 0, into
+// part_in) or dvar_r * [clamped row] (which = 1, into part_clamped; its CTAs exit at once unless some row was clamped,
+// so the rarely needed set costs no launch of its own).  Set 0 also accumulates b = sum_r dmu_r t_r.
 // ---------------------------------------------------------------------------------------------------
 constexpr int SY_KB = 32, SY_WARPS = 12, SY_STAGES = 3;     // SY_WARPS consumer warps (one 32 x 32 block each)
 constexpr int SY_CONS_THREADS = SY_WARPS * 32, SY_THREADS = SY_CONS_THREADS + 32;      // + one producer warp
@@ -1588,13 +1588,11 @@ __host__ __device__ inline size_t syrk_alpha_doubles(int MP, int nchunk) { retur
 __host__ __device__ inline int syrk_nblocks(int MP) { const int nb = MP / 32; return nb * (nb + 1) / 2; }
 
 __global__ void __launch_bounds__(SY_THREADS, 1)
-syrk_kernel(const double* __restrict__ T, const double* __restrict__ dvar, const double* __restrict__ craw, int which_in,
+syrk_kernel(const double* __restrict__ T, const double* __restrict__ dvar, const double* __restrict__ craw,
             int MP, long long R, int nchunk, double* __restrict__ part_in, const unsigned int* __restrict__ clamp_count,
             const double* __restrict__ dmu_in, double* __restrict__ part_alpha_in, double* __restrict__ part_clamped) {
-  // which_in == 2: both weight sets in one launch, blockIdx.z = which (the clamped-rows set, which is almost always
-  // skipped, then costs no launch of its own)
-  const int which = which_in == 2 ? (int)blockIdx.z : which_in;
-  double* __restrict__ part = (which_in == 2 && which == 1) ? part_clamped : part_in;
+  const int which = (int)blockIdx.z;
+  double* __restrict__ part = which == 1 ? part_clamped : part_in;
   const double* __restrict__ dmu = which == 0 ? dmu_in : nullptr;
   double* __restrict__ part_alpha = which == 0 ? part_alpha_in : nullptr;
   if (which == 1 && (clamp_count == nullptr || *clamp_count == 0u)) return;
@@ -1883,24 +1881,9 @@ int syrk_nchunk(int MP, long long R) {
 
 size_t syrk_part_doubles(int MP, long long R) { return (size_t)syrk_nblocks(MP) * syrk_nchunk(MP, R) * 1024; }
 
-// part: syrk_part_doubles(MP, R) doubles of scratch; part_alpha: syrk_alpha_doubles(MP, nchunk) doubles (which == 0 only)
-// the SYRK proper (DMMA-bound): per-chunk partial blocks into `part`, partial b into part_alpha (which == 0)
-int launch_syrk_main(const double* K, const double* dvar, const double* craw, int which, int MP, long long R,
-                     double* part, const unsigned int* clamp_count, const double* dmu, double* part_alpha,
-                     cudaStream_t st) {
-  const int nc = syrk_nchunk(MP, R);
-  const size_t smem = SY_STAGES * syrk_stage_doubles(MP) * sizeof(double);
-  static bool attr_done[kMaxDevices] = {false};
-  if (first_on_device(attr_done))
-    cudaFuncSetAttribute(syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)(SY_STAGES * syrk_stage_doubles(MAX_MP) * sizeof(double)));
-  dim3 grid(syrk_ngroups(MP), nc);
-  MOBO_LAUNCH("syrk_kernel", st, syrk_kernel<<<grid, SY_THREADS, smem, st>>>(K, dvar, craw, which, MP, R, nc, part, clamp_count,
-                                           which == 0 ? dmu : nullptr, which == 0 ? part_alpha : nullptr, nullptr));
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
-}
-
-// both weight sets (all rows -> part, clamped rows only -> part_clamped) in ONE launch
+// the SYRK proper (DMMA-bound), both weight sets (all rows -> part, clamped rows only -> part_clamped) in ONE launch:
+// per-chunk partial blocks, syrk_part_doubles(MP, R) doubles each, and partial b into part_alpha,
+// syrk_alpha_doubles(MP, syrk_nchunk(MP, R)) doubles
 int launch_syrk_both(const double* K, const double* dvar, const double* craw, int MP, long long R, double* part,
                      double* part_clamped, const unsigned int* clamp_count, const double* dmu, double* part_alpha,
                      cudaStream_t st) {
@@ -1911,7 +1894,7 @@ int launch_syrk_both(const double* K, const double* dvar, const double* craw, in
     cudaFuncSetAttribute(syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          (int)(SY_STAGES * syrk_stage_doubles(MAX_MP) * sizeof(double)));
   dim3 grid(syrk_ngroups(MP), nc, 2);
-  MOBO_LAUNCH("syrk_kernel", st, syrk_kernel<<<grid, SY_THREADS, smem, st>>>(K, dvar, craw, 2, MP, R, nc, part, clamp_count, dmu,
+  MOBO_LAUNCH("syrk_kernel", st, syrk_kernel<<<grid, SY_THREADS, smem, st>>>(K, dvar, craw, MP, R, nc, part, clamp_count, dmu,
                                            part_alpha, part_clamped));
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
@@ -1925,14 +1908,6 @@ int launch_syrk_reduce(int which, int MP, long long R, const double* part, doubl
   if (which == 0 && part_alpha && dalpha)
     MOBO_LAUNCH("reduce_partials_kernel", st, reduce_partials_kernel<<<(MP + 3) / 4, 128, 0, st>>>(part_alpha, nc * SY_ALPHA_PARTS, MP, MP, dalpha, 0));
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
-}
-
-int launch_syrk(const double* K, const double* dvar, const double* craw, int which, int MP, long long R,
-                double* part, double* A, const unsigned int* clamp_count, const double* dmu, double* part_alpha,
-                double* dalpha, double* clamp_flag_out, cudaStream_t st) {
-  const int e = launch_syrk_main(K, dvar, craw, which, MP, R, part, clamp_count, dmu, part_alpha, st);
-  if (e) return e;
-  return launch_syrk_reduce(which, MP, R, part, A, clamp_count, part_alpha, dalpha, clamp_flag_out, st);
 }
 
 }  // namespace mobo

@@ -11,8 +11,6 @@
 
 namespace mobo {
 
-constexpr int ST_MAX_LAYERS = 8;
-constexpr int ST_MAX_THETA = 5 + 2 * kMaxD;
 constexpr double kLog2Pi = 1.8378770664093454835606594728112;
 
 __device__ __forceinline__ double softplus_fwd(double x) { return x > 20.0 ? x : log1p(exp(x)); }   // torch softplus
@@ -26,16 +24,16 @@ __device__ __forceinline__ double sigmoid_fwd(double x) { return 1.0 / (1.0 + ex
 // ---- raw -> constrained parameters -----------------------------------------------------------------
 struct PrepArgs {
   int L, d;
-  const double* raw_theta[ST_MAX_LAYERS][ST_MAX_THETA];   // address of every raw hyper-parameter, theta order
-  const double* raw_noise[ST_MAX_LAYERS];
-  double noise_lo[ST_MAX_LAYERS], noise_hi[ST_MAX_LAYERS];
-  double* theta[ST_MAX_LAYERS];       // out: constrained, kernels' layout
+  const double* raw_theta[kMaxLayers][kMaxTheta];         // address of every raw hyper-parameter, theta order
+  const double* raw_noise[kMaxLayers];
+  double noise_lo[kMaxLayers], noise_hi[kMaxLayers];
+  double* theta[kMaxLayers];          // out: constrained, kernels' layout
   double* noise;                      // out: [L]
-  double* gops_scal[ST_MAX_LAYERS];   // scal block of each operator-gradient buffer
-  double* ops_scal[ST_MAX_LAYERS];    // scal block of each operator buffer (holds finalize_kernel's arrival counter)
+  double* gops_scal[kMaxLayers];      // scal block of each operator-gradient buffer
+  double* ops_scal[kMaxLayers];       // scal block of each operator buffer (zeroed here)
   unsigned int* clamp_count;          // [L]
   double dkl;                         // d loss / d KL = B / N
-  int* oc_flags[ST_MAX_LAYERS];       // block-to-block flags of the operator-chain kernel (256 ints), zeroed here
+  int* oc_flags[kMaxLayers];          // block-to-block flags of the operator-chain kernel (256 ints), zeroed here
 };
 
 __global__ void step_prep_kernel(const __grid_constant__ PrepArgs a) {
@@ -122,27 +120,27 @@ __global__ void __launch_bounds__(ELL_THREADS) ell_kernel(const __grid_constant_
 struct FinishArgs {
   int L, d, M, MP;
   double kl_scale;                       // B / N
-  const double* raw_theta[ST_MAX_LAYERS][ST_MAX_THETA];
-  double* g_raw_theta[ST_MAX_LAYERS][ST_MAX_THETA];
-  const double* dtheta_rows[ST_MAX_LAYERS];
-  const double* dtheta_pre[ST_MAX_LAYERS];
-  const double* dzf_rows[ST_MAX_LAYERS];   // layer l's d loss / d zf (zf_l = m_{l-1}); NULL for l = 0
-  const double* dzf_pre[ST_MAX_LAYERS];
-  const double* dm_pre[ST_MAX_LAYERS];
-  double* g_m[ST_MAX_LAYERS];
-  const double* raw_noise[ST_MAX_LAYERS];
-  double noise_lo[ST_MAX_LAYERS], noise_hi[ST_MAX_LAYERS];
-  double* g_raw_noise[ST_MAX_LAYERS];
-  const double* ell_part[ST_MAX_LAYERS];
-  int ell_blocks[ST_MAX_LAYERS];
-  const double* ops_scal[ST_MAX_LAYERS];
+  const double* raw_theta[kMaxLayers][kMaxTheta];
+  double* g_raw_theta[kMaxLayers][kMaxTheta];
+  const double* dtheta_rows[kMaxLayers];
+  const double* dtheta_pre[kMaxLayers];
+  const double* dzf_rows[kMaxLayers];      // layer l's d loss / d zf (zf_l = m_{l-1}); NULL for l = 0
+  const double* dzf_pre[kMaxLayers];
+  const double* dm_pre[kMaxLayers];
+  double* g_m[kMaxLayers];
+  const double* raw_noise[kMaxLayers];
+  double noise_lo[kMaxLayers], noise_hi[kMaxLayers];
+  double* g_raw_noise[kMaxLayers];
+  const double* ell_part[kMaxLayers];
+  int ell_blocks[kMaxLayers];
+  const double* ops_scal[kMaxLayers];
   double* out;                           // [0] loss, [1] KL * B / N, [2] data term, [3] status, [4] sticky status,
                                          // [5] sticky "loss not finite", [6] this step is bad (Adam skips), [7] retries
   int accumulate;
 };
 
 __global__ void __launch_bounds__(256) step_finish_kernel(const __grid_constant__ FinishArgs a) {
-  __shared__ double sdata[ST_MAX_LAYERS], sds2[ST_MAX_LAYERS];
+  __shared__ double sdata[kMaxLayers], sds2[kMaxLayers];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   // fold the per-block ELBO partials, one warp per layer, fixed order (lane-strided then butterfly)
   for (int l = warp; l < a.L; l += 8) {

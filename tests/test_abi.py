@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol():
     assert len(decl) >= 12
     for name in decl:
         assert hasattr(lib, name), name
-    assert lib.mobo_abi_version() == 102
+    assert lib.mobo_abi_version() == 103
 
 
 def test_ctypes_signatures_match_header():

@@ -87,6 +87,8 @@ def test_shape_limits_are_errors_not_wrong_numbers():
     # M > 256 and d > 8 are outside the kernels' limits
     rc = lib.mobo_layer_precompute(0, 2, 300, p, None, p, p, p, 1e-6, p, _lib.stream_ptr())
     assert rc == -2
+    rc = lib.mobo_layer_precompute_bwd(0, 2, 300, p, None, p, p, p, p, p, p, p, None, p, p, _lib.stream_ptr())
+    assert rc == -2
     rc = lib.mobo_layer_rows_fwd(0, 9, 16, p, None, p, p, p, 1, None, None, 1, None, 1, None, 4, 1, p, p, None, None,
                                  None, None, _lib.stream_ptr())
     assert rc == -2

@@ -21,7 +21,7 @@ int main(int argc, char** argv) {
   cudaMemcpy(dth1, th1.data(), th1.size() * 8, cudaMemcpyHostToDevice); cudaMemcpy(dm, m.data(), M * 8, cudaMemcpyHostToDevice); cudaMemcpy(dLq, Lq.data(), Lq.size() * 8, cudaMemcpyHostToDevice);
   LayerBatch b; b.n = nl; b.d = d; b.M = M; b.MP = MP;
   std::vector<double*> ops(nl);
-  for (int l = 0; l < MAX_BATCH; ++l) {
+  for (int l = 0; l < kMaxLayers; ++l) {
     const bool ok = l < nl;
     if (ok) { cudaMalloc(&ops[l], ops_size(MP) * 8); cudaMemset(ops[l], 0xff, ops_size(MP) * 8); }
     b.kind[l] = ok && l > 0 ? 1 : 0; b.Zx[l] = dZ; b.zf[l] = dm; b.theta[l] = (ok && l > 0) ? dth1 : dth0; b.m[l] = dm; b.Lq[l] = dLq; b.ops[l] = ok ? ops[l] : nullptr;

@@ -92,14 +92,15 @@ int main(int argc, char** argv) {
       else printf("  %-28s %8.1f us / iteration (%d launches)\n", a.name, us, a.c / iters);
     }
   }
-  {   // SYRK alone, with and without the b = sum dmu t accumulation of group 0
+  {   // SYRK alone, with and without the b = sum dmu t accumulation of set 0 (no clamp count: the clamped-rows set's
+      // CTAs exit at once, as in a step where no row was clamped)
     double* part; cudaMalloc(&part, (mobo::syrk_part_doubles(MP, R) + mobo::syrk_alpha_doubles(MP, mobo::syrk_nchunk(MP, R))) * 8);
     double* pal = part + mobo::syrk_part_doubles(MP, R);
     for (int variant = 0; variant < 2; ++variant) {
       float tt = 0;
       for (int it = 0; it < reps + 2; ++it) {
         cudaEventRecord(e[0]);
-        mobo::launch_syrk_main(Ts, dvar, craw, 0, MP, R, part, clamp, variant ? nullptr : dmu, pal, nullptr);
+        mobo::launch_syrk_both(Ts, dvar, craw, MP, R, part, nullptr, nullptr, variant ? nullptr : dmu, pal, nullptr);
         cudaEventRecord(e[1]); cudaEventSynchronize(e[1]);
         float x; cudaEventElapsedTime(&x, e[0], e[1]);
         if (it >= 2) tt += x;
