@@ -1,6 +1,5 @@
 // extern "C" entry points of libmobocmf_b200.so (declared in include/mobocmf_b200.h) and the host-side kernel
 // sequences behind them.
-#include <stdlib.h>
 #include <string.h>
 #include <mutex>
 #include "../../include/mobocmf_b200.h"
@@ -159,7 +158,7 @@ static void fill_row_args(RowArgs& a, int kind, int d, int M, const double* Zx, 
   a.mu = nullptr; a.var = nullptr; a.craw = nullptr; a.clamp_count = nullptr;
   a.Tsave = nullptr; a.Usave = nullptr;
   a.dmu = nullptr; a.dvar = nullptr; a.dk = nullptr; a.df = nullptr; a.dxrow = nullptr; a.part_theta = nullptr; a.part_zf = nullptr;
-  a.want_param_grads = 0; a.want_x_grads = 0;
+  a.want_param_grads = 0; a.want_x_grads = 0; a.sm_reserve = 0;
 }
 
 int mobo_layer_rows_fwd(int kind, int d, int M, const double* Zx, const double* zf, const double* theta,
@@ -227,7 +226,6 @@ static void fill_row_bwd_args(RowArgs& a, const double* dmu, const double* dvar,
   a.df = df; a.dxrow = dxrow;
   a.want_param_grads = want_param_grads; a.want_x_grads = dxrow != nullptr;
   if (!a.want_param_grads && !a.want_x_grads) a.want_param_grads = 1;
-  a.sm_reserve = 0;
 }
 
 int mobo_layer_rows_bwd(int kind, int d, int M, const double* Zx, const double* zf, const double* theta,
@@ -372,10 +370,6 @@ static bool g_side_stream_on = true;
 // side stream's operator-chain backward; measured on C4 (ms / step): round 1: 0 -> 2.84, 4 -> 2.72, 8 -> 2.71, 16 -> 2.75;
 // round-2 kernels: 0 -> 2.51, 4 -> 2.41, 8 -> 2.44, 12 -> 2.45, 16 -> 2.45
 constexpr int kSideStreamSMs = 4;
-static int side_stream_sms() {      // development override: MOBO_SIDE_SMS=n
-  static const int n = getenv("MOBO_SIDE_SMS") ? atoi(getenv("MOBO_SIDE_SMS")) : kSideStreamSMs;
-  return n;
-}
 void mobo_step_side_stream(int on) { g_side_stream_on = on != 0; }
 
 size_t mobo_elbo_step_workspace_doubles(int L, int d, int M, int S, long long B) {
@@ -397,6 +391,9 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
   const double* Zx[kMaxLayers]; const double* zf[kMaxLayers]; const double* theta[kMaxLayers];
   const double* m[kMaxLayers]; const double* Lq[kMaxLayers];
   double* ops[kMaxLayers]; double* dLq[kMaxLayers];
+  // the rows of each layer, which its forward and backward row passes both read: x itself at layer 0, above it x
+  // tiled S times, each row propagated from its sample of layer l - 1's q(f)
+  RowArgs rows[kMaxLayers];
   for (int l = 0; l < L; ++l) {
     const mobo_layer_desc& ld = D->layer[l];
     kinds[l] = l == 0 ? 0 : 1;
@@ -404,6 +401,9 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
     m[l] = ld.m; Lq[l] = ld.Lq;
     ops[l] = ws + y.ops[l];
     dLq[l] = (ld.g_Lq && !D->accumulate) ? ld.g_Lq : ws + y.dLq_tmp[l];
+    fill_row_args(rows[l], kinds[l], d, M, Zx[l], zf[l], theta[l], ops[l], D->x, l == 0 ? 1 : S,
+                  l == 0 ? nullptr : ws + y.mu[l - 1], l == 0 ? nullptr : ws + y.var[l - 1],
+                  l == 0 ? 1 : (int)(y.R[l] / y.R[l - 1]), ld.eps, y.R[l], nullptr, y.R[l], 1);
   }
   // 1. raw -> constrained
   {
@@ -425,12 +425,10 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
   MOBO_TRY(model_precompute(L, kinds, d, M, Zx, zf, theta, m, Lq, D->jitter, ops, st, false));
   // 3. forward row passes, low -> high fidelity
   for (int l = 0; l < L; ++l) {
-    const long long R = y.R[l];
-    MOBO_TRY(mobo_layer_rows_fwd(kinds[l], d, M, Zx[l], zf[l], theta[l], ops[l], D->x, l == 0 ? 1 : S,
-                                 l == 0 ? nullptr : ws + y.mu[l - 1], l == 0 ? nullptr : ws + y.var[l - 1],
-                                 l == 0 ? 1 : (int)(R / y.R[l - 1]), D->layer[l].eps, R, nullptr, R, 1,
-                                 ws + y.mu[l], ws + y.var[l], ws + y.craw[l], clamp + l, ws + y.Ts[l], ws + y.Us[l],
-                                 stream));
+    RowArgs a = rows[l];
+    a.mu = ws + y.mu[l]; a.var = ws + y.var[l]; a.craw = ws + y.craw[l]; a.clamp_count = clamp + l;
+    a.Tsave = ws + y.Ts[l]; a.Usave = ws + y.Us[l];
+    MOBO_TRY(launch_row_fwd(a, st));
   }
   // 4. ELBO terms and backward row passes, high -> low fidelity.  Per layer the main stream runs the SYRK statistics,
   //    the product and the covariance-gradient kernels; that layer's operator-chain backward (a dozen latency-bound
@@ -464,14 +462,11 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
     // its all-reduce now, behind the lower layers' row kernels (mobo_step_ctx_wait_layer)
     if (scp && !D->accumulate && cudaEventRecord(sc.done[l], ss) != cudaSuccess) return -1;
     // main stream: dk = W^T dt and the covariance gradient
-    RowArgs a;
-    fill_row_args(a, kinds[l], d, M, Zx[l], zf[l], theta[l], ops[l], D->x, l == 0 ? 1 : S,
-                  l == 0 ? nullptr : ws + y.mu[l - 1], l == 0 ? nullptr : ws + y.var[l - 1],
-                  l == 0 ? 1 : (int)(R / y.R[l - 1]), D->layer[l].eps, R, nullptr, R, 1);
+    RowArgs a = rows[l];
     fill_row_bwd_args(a, ws + y.dmu[l], ws + y.dvar[l], ws + y.craw[l], ws + y.Ts[l], ws + y.Us[l], 1, ws + y.df[l],
                       nullptr);
     a.clamp_count = clamp + l;
-    a.sm_reserve = fork ? side_stream_sms() : 0;
+    a.sm_reserve = fork ? kSideStreamSMs : 0;
     MOBO_TRY(rows_bwd_main(a, kinds[l], d, M, R, ws + y.rows_work, ws + y.kg_part[l], ws + y.dtheta_rows[l],
                            l == 0 ? nullptr : ws + y.dzf_rows[l], st, fork ? ss : nullptr, fork ? sc.kg[l] : nullptr));
   }

@@ -144,7 +144,6 @@ struct CovSmem {
 
 struct RowSmem : CovSmem<ROW_WARPS, false> {
   double red[3][NCH_MAX][TR];     // per warp-pair partial column sums: q1, mu, q2
-  int xsel[TR];                   // tile-shared covariance build: which of the tile's distinct x rows a tile row reads
 };
 static_assert(ROW_WARPS * RPW == TR, "the covariance build maps RPW rows to each warp of the row tile");
 
@@ -217,32 +216,6 @@ __device__ __forceinline__ void store_acc_rows(const double (&acc)[2][2][4][2], 
   }
 }
 
-// loads the rows of one tile: x, propagated input f (sample of the previous layer's q(f), the fused
-// reparameterised propagation of layers/mfdgp_hidden_layer.py:263-274), k_xx
-template <class SM>
-__device__ __forceinline__ void load_tile_rows(const RowArgs& a, SM& sm, long long row0, int nvalid) {
-  const int tid = threadIdx.x;
-  for (int idx = tid; idx < SM::ROWS * a.d; idx += SM::THREADS) {
-    const int r = idx / a.d, c = idx - r * a.d;
-    sm.xs[r][c] = r < nvalid ? a.x[(size_t)((row0 + r) / a.xrep) * a.d + c] : 0.0;
-  }
-  if (tid < SM::ROWS) {
-    double f = 0.0;
-    if (tid < nvalid && a.kind == 1) {
-      const long long row = row0 + tid;
-      if (a.f_direct) {
-        f = a.f_direct[row];
-      } else {
-        const long long pr = row / a.prep;
-        const double vp = fmax(a.var_prev[pr], kMinVariance);
-        f = a.mu_prev[pr] + sqrt(vp) * a.eps[row % a.eps_mod];
-      }
-    }
-    sm.fs[tid] = f;
-    sm.kxx[tid] = sm.kf.kind == 0 ? sm.kf.a1 : sm.kf.a1 * (sm.kf.vlin * f * f + sm.kf.af) + sm.kf.a2;
-  }
-}
-
 __device__ inline void load_kern_fast(KernFast& kf, int kind, int d, const double* __restrict__ theta) {
   const double nhl2e = -0.5 * 1.4426950408889634074;     // -1/2 log2(e)
   kf.kind = kind; kf.d = d;
@@ -265,15 +238,14 @@ __device__ inline void load_kern_fast(KernFast& kf, int kind, int d, const doubl
 }
 
 template <class SM>
-__device__ __forceinline__ void load_inducing(const RowArgs& a, SM& sm, bool with_zx = true) {
+__device__ __forceinline__ void load_inducing(const RowArgs& a, SM& sm) {
   const int tid = threadIdx.x;
   if (tid == 0) load_kern_fast(sm.kf, a.kind, a.d, a.theta);
   fill_exp2_tab(sm.e2tab, tid, SM::THREADS);
-  if (with_zx)
-    for (int idx = tid; idx < a.MP * a.d; idx += SM::THREADS) {
-      const int j = idx / a.d, c = idx - j * a.d;
-      sm.zsT[c][j] = j < a.M ? a.Zx[(size_t)j * a.d + c] : 0.0;
-    }
+  for (int idx = tid; idx < a.MP * a.d; idx += SM::THREADS) {
+    const int j = idx / a.d, c = idx - j * a.d;
+    sm.zsT[c][j] = j < a.M ? a.Zx[(size_t)j * a.d + c] : 0.0;
+  }
   for (int j = tid; j < a.MP; j += SM::THREADS) sm.zfs[j] = (a.kind == 1 && j < a.M) ? a.zf[j] : 0.0;
 }
 
@@ -358,8 +330,7 @@ __device__ __forceinline__ bool warp_rows_share_x(const RowArgs& a, long long ro
 
 // The general covariance build of the forward kernel (layer 0, and upper layers whose rows do not share x in large
 // groups: single-sample training, small S).  Kept out of line: its per-dimension register arrays (up to 8 dimensions
-// x 4 rows) would otherwise set the register allocation of the whole kernel, whose hot configuration (xshare, below)
-// needs none of them.
+// x 4 rows) would otherwise set the register allocation of the whole kernel, whose DMMA products need none of them.
 __device__ __noinline__ void build_k_tile_generic(const RowArgs& a, const RowSmem& sm, double* Ks, int ldb, unsigned row0,
                                                   int nvalid, int warp, int lane) {
   if (a.kind == 0) build_k_tile_d<0, false>(sm, Ks, ldb, a.M, a.MP, nvalid, warp, lane);
@@ -436,18 +407,11 @@ __device__ __forceinline__ const double2* frag_start(const double* Af, int MP, i
   return reinterpret_cast<const double2*>(Af) + ((size_t)s * (MP >> 2) + (upper ? 4 * s : 0)) * 32 + lane;
 }
 
-// Distinct x rows a 32-row tile may hold for the tile-shared covariance build (below); xrep >= 11 guarantees it
-constexpr int XMAX = 4, XSHARE_MIN_REP = 11;
-
-// Forward row pass.  Per 32-row tile (two CTAs per SM, 8 warps each):
-//   rows (prefetched one tile ahead into registers) -> shared;  K(Z_l, rows) into the tile buffer;  t = W k (DMMA);
-//   t -> tile buffer (bulk-stored to Tsave from there);  u = H^T t (DMMA), stored from the accumulators;  mean / variance.
-// Covariance build when the rows are MC samples of few points (xrep >= 11: at most XMAX = 4 distinct x per tile; the
-// S = 64 training tiles have one, the S = 25 acquisition tiles two or three): the two x-kernels a1 E1, a2 E2 depend on
-// (x, z_j) only, so thread j evaluates them ONCE per tile and distinct x into shared memory, and the per-(row, j) work
-// shrinks to the f-kernel: one exponential instead of three (and no per-dimension arithmetic).  In the first version
-// every warp re-evaluated them for its own 4 rows (8x redundant at S = 64) and the build - DFMA work on the FP64 pipe
-// the co-resident CTA's DMMAs are hogging - was 30 % of a CTA's time (tools/row_bench -DROW_TIMING).
+// Forward row pass of the rows that are not MC samples of few points (layer 0, single-sample training, small S; the
+// others go to row_fwd_ws_kernel below).  Per 32-row tile (two CTAs per SM, 8 warps each):
+//   row data (prefetched one tile ahead into registers) and x -> shared;  K(Z_l, rows) into the tile buffer
+//   (build_k_tile_generic);  t = W k (DMMA);  t -> tile buffer (bulk-stored to Tsave from there);  u = H^T t (DMMA),
+//   stored from the accumulators;  mean / variance.
 __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(const __grid_constant__ RowArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   RowSmem& sm = *reinterpret_cast<RowSmem*>(smem_raw);
@@ -463,14 +427,9 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(c
   const double* W = a.ops + ops_block(MP, OPS_WF);
   const double* G = a.ops + ops_block(MP, OPS_HTF);
   const double* beta = a.ops + ops_beta(MP);
-  // tile-shared covariance build: decided per launch (the shared x-kernel values live where the legacy build keeps Z^T)
-  const bool xshare = a.kind == 1 && a.xrep >= XSHARE_MIN_REP;
-  double (*s1s)[MAX_MP] = sm.zsT;            // [XMAX][MAX_MP]  a1 E1(x_c, z_j)
-  double (*s2s)[MAX_MP] = sm.zsT + XMAX;     // [XMAX][MAX_MP]  a2 E2(x_c, z_j)
-  static_assert(2 * XMAX <= kMaxD, "the shared x-kernel values overlay zsT");
 
   RT_DECL
-  load_inducing(a, sm, !xshare);
+  load_inducing(a, sm);
   double bi[2][2] = {{0.0, 0.0}, {0.0, 0.0}};
   if (active) {
 #pragma unroll
@@ -479,34 +438,25 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(c
       for (int ib = 0; ib < 2; ++ib) bi[sl][ib] = __ldg(beta + 16 * (sl == 0 ? sA : sB) + 8 * ib + g);
   }
 
-  // ---- row data, prefetched one tile ahead: threads 0..31 hold a row's (mean, variance, normal) or its direct f,
-  //      threads 32.. one coordinate of one of the tile's distinct x rows (xshare) ----
+  // ---- row data, prefetched one tile ahead: threads 0..31 hold a row's (mean, variance, normal) or its direct f ----
   // (row indices are 32-bit here: the launcher refuses R >= 2^31, callers chunk long before that)
   const unsigned R = (unsigned)a.R, ntiles = (R + TR - 1) / TR;
   const unsigned uxrep = (unsigned)a.xrep, uprep = (unsigned)a.prep;
   const unsigned ueps = a.eps_mod >= a.R ? 0u : (unsigned)a.eps_mod;       // 0: eps index == row
   double pf_a = 0.0, pf_b = 1.0, pf_c = 0.0;
   auto prefetch = [&](unsigned tile) {
-    if (tile >= ntiles) return;
-    const unsigned row0 = tile * TR;
-    if (tid < TR) {
-      const unsigned row = row0 + tid;
-      pf_a = 0.0; pf_b = 1.0; pf_c = 0.0;
-      if (row < R && a.kind == 1) {
-        if (a.f_direct) {
-          pf_a = a.f_direct[row];
-        } else {
-          const unsigned pr = row / uprep;
-          pf_a = a.mu_prev[pr];
-          pf_b = a.var_prev[pr];
-          pf_c = a.eps[ueps ? row % ueps : row];
-        }
+    if (tile >= ntiles || tid >= TR) return;
+    const unsigned row = tile * TR + tid;
+    pf_a = 0.0; pf_b = 1.0; pf_c = 0.0;
+    if (row < R && a.kind == 1) {
+      if (a.f_direct) {
+        pf_a = a.f_direct[row];
+      } else {
+        const unsigned pr = row / uprep;
+        pf_a = a.mu_prev[pr];
+        pf_b = a.var_prev[pr];
+        pf_c = a.eps[ueps ? row % ueps : row];
       }
-    } else if (xshare && tid < TR + XMAX * a.d) {
-      const int c = (tid - TR) / a.d, cc = (tid - TR) - c * a.d;
-      const unsigned xi = row0 / uxrep + c;
-      const unsigned last = min(R - 1, row0 + TR - 1) / uxrep;
-      pf_a = xi <= last ? a.x[(size_t)xi * a.d + cc] : 0.0;
     }
   };
   prefetch(blockIdx.x);
@@ -522,78 +472,22 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(c
   for (unsigned tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const unsigned row0 = tile * TR;
     const int nvalid = (int)min((unsigned)TR, R - row0);
-    const unsigned xi0 = row0 / uxrep;
     // ---- this tile's rows: registers -> shared ----
     if (tid < TR) {
       double f = 0.0;
       if (tid < nvalid && a.kind == 1) f = a.f_direct ? pf_a : pf_a + sqrt(fmax(pf_b, kMinVariance)) * pf_c;
       sm.fs[tid] = f;
       sm.kxx[tid] = sm.kf.kind == 0 ? sm.kf.a1 : sm.kf.a1 * (sm.kf.vlin * f * f + sm.kf.af) + sm.kf.a2;
-      sm.xsel[tid] = tid < nvalid ? (int)((row0 + tid) / uxrep - xi0) : 0;
-    } else if (xshare) {
-      if (tid < TR + XMAX * a.d) { const int c = (tid - TR) / a.d; sm.xs[c][(tid - TR) - c * a.d] = pf_a; }
     }
-    if (!xshare) {
-      for (int idx = tid; idx < TR * a.d; idx += ROW_THREADS) {
-        const int r = idx / a.d, c = idx - r * a.d;
-        sm.xs[r][c] = r < nvalid ? a.x[(size_t)((row0 + r) / uxrep) * a.d + c] : 0.0;
-      }
+    for (int idx = tid; idx < TR * a.d; idx += ROW_THREADS) {
+      const int r = idx / a.d, c = idx - r * a.d;
+      sm.xs[r][c] = r < nvalid ? a.x[(size_t)((row0 + r) / uxrep) * a.d + c] : 0.0;
     }
     __syncthreads();
     prefetch(tile + gridDim.x);         // lands during the products
     RT_TICK(1);
     // ---- K(Z_l, rows) into shared memory ----
-    if (xshare) {
-      // (a) thread j: a1 E1 and a2 E2 between inducing point j and each distinct x of the tile
-      const int nx = (int)((row0 + nvalid - 1) / uxrep - xi0) + 1;
-      if (tid < MP) {
-        const KernFast& kf = sm.kf;
-        const bool jok = tid < a.M;
-        double D1[XMAX], D2[XMAX];
-#pragma unroll
-        for (int q = 0; q < XMAX; ++q) { D1[q] = kf.la1; D2[q] = kf.la2; }
-        for (int c = 0; c < a.d; ++c) {          // dimensions in ascending order, like every other build of K
-          const double z = jok ? __ldg(a.Zx + (size_t)tid * a.d + c) : 0.0;
-          const double2 cc = kf.cc[c];
-#pragma unroll
-          for (int q = 0; q < XMAX; ++q)
-            if (q < nx) {
-              const double df = sm.xs[q][c] - z;
-              const double d2 = df * df;
-              D1[q] = fma(d2, cc.x, D1[q]);
-              D2[q] = fma(d2, cc.y, D2[q]);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < XMAX; ++q)
-          if (q < nx) {
-            s1s[q][tid] = jok ? exp2_tab(D1[q], sm.e2tab) : 0.0;
-            s2s[q][tid] = jok ? exp2_tab(D2[q], sm.e2tab) : 0.0;
-          }
-      }
-      __syncthreads();
-      // (b) warp <-> RPW rows, lane <-> inducing point of a 32-chunk: k = s1 (v f z_f + a_f E_f) + s2
-      const KernFast& kf = sm.kf;
-      const int rbase = warp * RPW;
-      double f[RPW], vf[RPW];
-      int xs_[RPW];
-#pragma unroll
-      for (int i = 0; i < RPW; ++i) { f[i] = sm.fs[rbase + i]; vf[i] = kf.vlin * f[i]; xs_[i] = sm.xsel[rbase + i]; }
-      const double laf = kf.laf, cf = kf.cf;
-      for (int ch = 0; ch < MP / 32; ++ch) {
-        const int j = 32 * ch + lane;
-        const double zf = sm.zfs[j];
-#pragma unroll
-        for (int i = 0; i < RPW; ++i) {
-          const double dff = f[i] - zf;
-          const double Ef = exp2_tab(fma(dff * dff, cf, laf), sm.e2tab);
-          const double k = fma(s1s[xs_[i]][j], fma(vf[i], zf, Ef), s2s[xs_[i]][j]);
-          Ks[(size_t)(rbase + i) * ldb + j] = rbase + i < nvalid ? k : 0.0;
-        }
-      }
-    } else {
-      build_k_tile_generic(a, sm, Ks, ldb, row0, nvalid, warp, lane);
-    }
+    build_k_tile_generic(a, sm, Ks, ldb, row0, nvalid, warp, lane);
     RT_TICK(2);
     __syncthreads();
     RT_TICK(3);
@@ -704,7 +598,13 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(c
 
 // ---------------------------------------------------------------------------------------------------------------
 // Warp-specialised forward kernel: the hot configuration (upper layers whose rows are MC samples of few points: the
-// S-sample training tiles and the acquisition tiles; `xshare`).
+// S-sample training tiles and the acquisition tiles).
+//
+// Sample-shared covariance build: with xrep >= XSHARE_MIN_REP = 11 a 32-row tile holds at most XMAX = 4 distinct x (the
+// S = 64 training tiles one, the S = 25 acquisition tiles two or three).  The two x-kernels a1 E1, a2 E2 depend on
+// (x, z_j) only, so they are evaluated ONCE per tile and distinct x, and the per-(row, j) work shrinks to the f-kernel:
+// one exponential instead of three, and no per-dimension arithmetic.  At S = 64 that is 8x fewer x-kernel evaluations
+// than build_k_tile's one per warp of RPW rows.
 //
 // What the measurements said (tools/row_bench -DROW_TIMING, profiles/r02_row_fwd_phases.txt):
 //  * DFMA and DMMA share the FP64 pipe and the schedulers arbitrate between warps, not work: next to warps that stream
@@ -733,6 +633,7 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_CTAS_PER_SM) row_fwd_kernel(c
 // symmetric support warps that own two rows of every tile for build, sums and stores; the product warps building a
 // quarter of K themselves between two tiles.
 // ---------------------------------------------------------------------------------------------------------------
+constexpr int XMAX = 4, XSHARE_MIN_REP = 11;     // distinct x rows per tile, and the xrep that bounds them by XMAX
 constexpr int WS_PROD_WARPS = ROW_WARPS, WS_BUILD_WARPS = 16, WS_FIN_WARPS = 4;
 constexpr int WS_PROD_THREADS = WS_PROD_WARPS * 32, WS_BUILD_THREADS = WS_BUILD_WARPS * 32, WS_FIN_THREADS = WS_FIN_WARPS * 32;
 constexpr int WS_THREADS = WS_PROD_THREADS + WS_BUILD_THREADS + WS_FIN_THREADS;      // 896: launched with 72 registers
@@ -1780,16 +1681,10 @@ static bool first_on_device(bool (&done)[kMaxDevices]) {
 
 int row_grid(long long R) {
   const long long ntiles = (R + TR - 1) / TR;
-#ifdef ROW_TIMING
-  static const int dbg_ctas = getenv("MOBO_ROW_CTAS") ? atoi(getenv("MOBO_ROW_CTAS")) : ROW_CTAS_PER_SM;   // tools/row_bench
-  const long long cap = (long long)num_sms() * dbg_ctas;
-#else
   const long long cap = (long long)num_sms() * ROW_CTAS_PER_SM;
-#endif
   return (int)(ntiles < cap ? (ntiles > 0 ? ntiles : 1) : cap);
 }
 
-static bool g_row_fwd_pingpong = true;      // tools: compare against the two-CTA kernel
 int launch_row_fwd(const RowArgs& a, cudaStream_t st) {
   if (a.MP % 32 != 0 || a.MP > MAX_MP || a.d > kMaxD || a.M > a.MP) return -2;
   if (a.R >= (1ll << 31) - TR) return -2;      // 32-bit row indices in the kernel; callers chunk (MFDGP.ACQ_CHUNK)
@@ -1801,10 +1696,7 @@ int launch_row_fwd(const RowArgs& a, cudaStream_t st) {
   if (first_on_device(attr_done_ws))
     cudaFuncSetAttribute(row_fwd_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws_smem_bytes(MAX_MP));
   if (a.R <= 0) return 0;
-#ifdef ROW_TIMING
-  g_row_fwd_pingpong = getenv("MOBO_NO_PP") == nullptr;
-#endif
-  if (a.kind == 1 && a.xrep >= XSHARE_MIN_REP && g_row_fwd_pingpong) {
+  if (a.kind == 1 && a.xrep >= XSHARE_MIN_REP) {
     // rows are MC samples of few points (S-sample training, acquisition): the warp-specialised kernel, one CTA per SM
     if ((a.Tsave && ((uintptr_t)a.Tsave & 15)) || (a.Usave && ((uintptr_t)a.Usave & 15))) return -2;   // bulk copies
     const long long ntiles = (a.R + TR - 1) / TR;

@@ -130,11 +130,11 @@ int main(int argc, char** argv) {
     const char* names[12] = {"load_inducing (once)", "load_tile_rows+sync", "build K", "sync after build", "gemm1 (warp 0)",
                              "sums after gemm1", "sync (K free)", "t -> tile + sync", "gemm2 (warp 0)", "sums + U stores",
                              "sync", "epilogue + bulk wait + sync"};
-    const bool pp = getenv("MOBO_NO_PP") == nullptr && S >= 11;   // product warps of the warp-specialised kernel
+    const bool pp = S >= mobo::XSHARE_MIN_REP;   // product warps of the warp-specialised kernel
     const char* pp_names[12] = {"setup (once)", "WAIT: K ready", "gemm1 (warp 0)", "sync, t -> tile, sync, signal",
                                 "gemm2 (warp 0)", "WAIT: t sums / store done", "u -> tile, sync, signal", "-", "-", "-", "-", "-"};
     if (pp) for (int k = 0; k < 12; ++k) names[k] = pp_names[k];
-    const int grid = pp ? 148 : 148 * (getenv("MOBO_ROW_CTAS") ? atoi(getenv("MOBO_ROW_CTAS")) : 2);
+    const int grid = pp ? 148 : 148 * mobo::ROW_CTAS_PER_SM;
     double tot = 0, s[12] = {0};
     for (int b = 0; b < grid; ++b) for (int k = 0; k < 12; ++k) { s[k] += (double)t[0][b][k]; tot += (double)t[0][b][k]; }
     printf("forward kernel (training launch: saves t / u), cycles of thread 0 summed over %d CTAs: share per phase\n", grid);
