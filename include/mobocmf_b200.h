@@ -178,7 +178,27 @@ int mobo_acq_moments(int fidelity, int d, int M, int S, long long n, const doubl
                      const double* const* theta, const double* const* ops, const double* const* samples,
                      const double* raw_noise, double noise_lower, double noise_upper, const double* X,
                      double* out_mu, double* out_var, double* scratch, void* stream);
-/* out[i] (+)= 1/2 max(0, log vu[i] - log vc[i])   (_JES_MFDGP.forward, acquisition_functions/JESMOC_MFDGP.py:52) */
+/* Backward of mobo_acq_moments: d / dX of the acquisition chain for optimize_acqf, which differentiates
+ * _JES_MFDGP.forward with respect to the candidates (MFDGP.predict_for_acquisition, mobocmf/models/mfdgp.py:237-262;
+ * acquisition_functions/JESMOC_MFDGP.py:38-52,142-143).  Same inputs as mobo_acq_moments plus the upstream gradients
+ * d_mu[n], d_var[n] (either NULL: zero).  Outputs dX[n x d] and, when d_raw_noise != NULL, d_raw_noise[1]
+ * (d / d raw_noise of the likelihood, the one parameter the eval-mode chain does not hold constant); accumulate = 1
+ * adds to both instead of overwriting them.  Stateless: it recomputes the forward with exactly mobo_acq_moments'
+ * arguments (so its moments are bit-identical to the caller's), saving t and u of every layer in `work`, then runs
+ * the row backward of every layer; the result is deterministic (fixed summation orders, no atomics).
+ * work: mobo_acq_bwd_work_doubles(...) doubles, 16-byte aligned, laid out as these regions in order, each starting
+ * at a multiple of 16 doubles, with R_0 = n, R_l = n S (l >= 1), F = fidelity, B(R) = mobo_rows_save_doubles(M, R):
+ *   for l = 0 .. F: mu_l[R_l], var_l[R_l], T_l[B(R_l)], U_l[B(R_l)], dxrow_l[R_l d];
+ *   then dmu[R_F], dvar[R_F], df[R_F], dk[B(R_F)], noise partials[ceil(n / 256)].
+ * Returns -2 (before any launch) for fidelity outside [0, 8), d outside [1, 8], M outside [1, 256], S < 1, n < 1 or
+ * n S >= 2^31 - 32; mobo_acq_bwd_work_doubles returns 0 for those. */
+size_t mobo_acq_bwd_work_doubles(int fidelity, int d, int M, int S, long long n);
+int mobo_acq_moments_bwd(int fidelity, int d, int M, int S, long long n, const double* Zx,
+                         const double* const* zf, const double* const* theta, const double* const* ops,
+                         const double* const* samples, const double* raw_noise, double noise_lower,
+                         double noise_upper, const double* X, const double* d_mu, const double* d_var,
+                         int accumulate, double* dX, double* d_raw_noise, double* work, void* stream);
+/* out[i] (+)=1/2 max(0, log vu[i] - log vc[i])   (_JES_MFDGP.forward, acquisition_functions/JESMOC_MFDGP.py:52) */
 int mobo_jes(const double* var_uncond, const double* var_cond, long long n, int accumulate, double* out, void* stream);
 
 /* ---- Pareto-sample generation (SURVEY.md section 8f-3) ----

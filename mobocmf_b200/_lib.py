@@ -46,6 +46,9 @@ _SIGNATURES = {
     "mobo_adam_tick": (_c_i, [_c_dp, _c_dp, _c_dp]),
     "mobo_acq_moments": (_c_i, [_c_i, _c_i, _c_i, _c_i, _c_ll, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_d, _c_d,
                                 _c_dp, _c_dp, _c_dp, _c_dp, _c_dp]),
+    "mobo_acq_bwd_work_doubles": (_c_sz, [_c_i, _c_i, _c_i, _c_i, _c_ll]),
+    "mobo_acq_moments_bwd": (_c_i, [_c_i, _c_i, _c_i, _c_i, _c_ll, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_dp, _c_d,
+                                    _c_d, _c_dp, _c_dp, _c_dp, _c_i, _c_dp, _c_dp, _c_dp, _c_dp]),
     "mobo_jes": (_c_i, [_c_dp, _c_dp, _c_ll, _c_i, _c_dp, _c_dp]),
     # Pareto-sample generation
     "mobo_rff_eval": (_c_i, [_c_i, _c_i, _c_i, _c_dp, _c_dp, _c_dp, _c_ll, _c_dp, _c_dp, _c_dp]),

@@ -27,6 +27,8 @@ class _JES_MFDGP(torch.nn.Module):
         with settings.num_likelihood_samples(1):
             _, pred_variances_cond = self.mfdgp_cond.predict_for_acquisition(X, self.fidelity)
         self.mfdgp_cond.train()
+        # with X.requires_grad the variances carry a graph and the JES term is torch arithmetic over two n-vectors; on
+        # the fused chain that graph holds X, not the chain's rows (its backward recomputes them, mobo_acq_moments_bwd)
         if not (pred_variances_uncond.requires_grad or pred_variances_cond.requires_grad) and \
                 pred_variances_uncond.is_cuda:
             from .. import _lib
@@ -161,8 +163,10 @@ def jes_sweep(X: Tensor, fidelity: int, blackboxes, chunk: int = 1 << 17) -> Ten
 
     ``blackboxes``: one ``(uncond MFDGP, [cond MFDGP of Pareto sample p, ...])`` pair per objective / constraint.
     X: (n, d) or (n, 1, d) fp64 CUDA.  Without gradients every model chain is ONE enqueue of the fused acquisition
-    kernels (``mobo_acq_moments`` + ``mobo_jes``), candidates in chunks that bound the n * S scratch; with
-    ``X.requires_grad`` the composable autograd path provides d acq / dX (what optimize_acqf consumes).
+    kernels (``mobo_acq_moments`` + ``mobo_jes``), candidates in chunks of ``chunk`` that bound the n * S scratch.
+    With ``X.requires_grad`` the same fused chain is differentiable (what optimize_acqf consumes): its backward
+    recomputes each model's rows in chunks of ``MFDGP.ACQ_GRAD_CHUNK`` candidates (``mobo_acq_moments_bwd``), so a
+    chain keeps O(n) memory, a few doubles per candidate, between the forward and the backward.
     Candidates are independent: shard X across GPUs with ``util.distributed.shard_bounds``, no collective."""
     from .. import _lib
     if X.dim() > 2:

@@ -535,6 +535,19 @@ int mobo_adam_tick(long long* step_dev, const double* skip_flag, void* stream) {
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
+// the rows of layer l of the acquisition chain, which mobo_acq_moments and the forward recomputed by
+// mobo_acq_moments_bwd both read: the n candidates at layer 0, above it row i*S+s = (candidate i, sample s), its
+// propagated input from row i (layer 1) or row i*S+s (layers >= 2) of the layer below, eval mode
+static void fill_acq_row_args(RowArgs& a, int l, int d, int M, int S, long long n, const double* Zx,
+                              const double* const* zf, const double* const* theta, const double* const* ops,
+                              const double* const* samples, const double* X, const double* mu_prev,
+                              const double* var_prev) {
+  const long long R = l == 0 ? n : n * (long long)S;
+  fill_row_args(a, l == 0 ? 0 : 1, d, M, Zx, l == 0 ? nullptr : zf[l], theta[l], ops[l], X, l == 0 ? 1 : S,
+                l == 0 ? nullptr : mu_prev, l == 0 ? nullptr : var_prev, l == 1 ? S : 1,
+                l == 0 ? nullptr : samples[l], S, nullptr, R, 0);
+}
+
 int mobo_acq_moments(int fidelity, int d, int M, int S, long long n, const double* Zx, const double* const* zf,
                      const double* const* theta, const double* const* ops, const double* const* samples,
                      const double* raw_noise, double noise_lower, double noise_upper, const double* X,
@@ -544,15 +557,12 @@ int mobo_acq_moments(int fidelity, int d, int M, int S, long long n, const doubl
   const long long RS = n * (long long)S;
   double* mu[2] = {scratch, scratch + 2 * RS};
   double* var[2] = {scratch + RS, scratch + 3 * RS};
-  long long Rprev = n;
   for (int l = 0; l <= fidelity; ++l) {
-    const long long R = l == 0 ? n : RS;
     const int cur = l & 1, prv = cur ^ 1;
-    MOBO_TRY(mobo_layer_rows_fwd(l == 0 ? 0 : 1, d, M, Zx, l == 0 ? nullptr : zf[l], theta[l], ops[l], X,
-                                 l == 0 ? 1 : S, l == 0 ? nullptr : mu[prv], l == 0 ? nullptr : var[prv],
-                                 l == 0 ? 1 : (int)(R / Rprev), l == 0 ? nullptr : samples[l], S, nullptr, R, 0,
-                                 mu[cur], var[cur], nullptr, nullptr, nullptr, nullptr, stream));
-    Rprev = R;
+    RowArgs a;
+    fill_acq_row_args(a, l, d, M, S, n, Zx, zf, theta, ops, samples, X, mu[prv], var[prv]);
+    a.mu = mu[cur]; a.var = var[cur];
+    MOBO_TRY(launch_row_fwd(a, st));
   }
   MomentArgs a;
   a.n = n; a.S = S; a.tiled = fidelity >= 1 ? 1 : 0;
@@ -560,6 +570,107 @@ int mobo_acq_moments(int fidelity, int d, int M, int S, long long n, const doubl
   a.noise_lo = noise_lower; a.noise_hi = noise_upper; a.raw_noise = raw_noise;
   a.out_mu = out_mu; a.out_var = out_var;
   MOBO_LAUNCH("moment_kernel", st, moment_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a));
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// backward of the acquisition chain: recompute the chunk's forward with t and u saved, then the row backward of
+// every layer, high -> low, and the fold of d / dX
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+struct AcqBwdLayout {
+  size_t mu[kMaxLayers], var[kMaxLayers], Ts[kMaxLayers], Us[kMaxLayers], dxrow[kMaxLayers];
+  size_t dmu, dvar, df, dk, noise_part, total;
+  int noise_blocks;
+};
+
+bool acq_bwd_shape_ok(int fidelity, int d, int M, int S, long long n) {
+  return fidelity >= 0 && fidelity < kMaxLayers && d >= 1 && d <= kMaxD && M >= 1 && padded(M) <= MAX_MP && S >= 1 &&
+         n >= 1 && n < kMaxRows && n * (long long)S < kMaxRows;
+}
+
+// every region starts at a multiple of 16 doubles (the bulk copies of the row kernels need 16-byte aligned T / U
+// rows); the order is the one include/mobocmf_b200.h documents
+AcqBwdLayout acq_bwd_layout(int fidelity, int d, int M, int S, long long n) {
+  AcqBwdLayout y;
+  size_t off = 0;
+  auto take = [&](size_t k) { const size_t o = off; off += (k + 15) / 16 * 16; return o; };
+  const long long RF = fidelity == 0 ? n : n * (long long)S;
+  for (int l = 0; l <= fidelity; ++l) {
+    const long long R = l == 0 ? n : n * (long long)S;
+    y.mu[l] = take(R); y.var[l] = take(R);
+    y.Ts[l] = take(mobo_rows_save_doubles(M, R)); y.Us[l] = take(mobo_rows_save_doubles(M, R));
+    y.dxrow[l] = take((size_t)R * d);
+  }
+  y.dmu = take(RF); y.dvar = take(RF); y.df = take(RF);
+  y.dk = take(mobo_rows_save_doubles(M, RF));
+  y.noise_blocks = (int)((n + ACQ_THREADS - 1) / ACQ_THREADS);
+  y.noise_part = take(y.noise_blocks);
+  y.total = off;
+  return y;
+}
+
+}  // namespace
+
+size_t mobo_acq_bwd_work_doubles(int fidelity, int d, int M, int S, long long n) {
+  if (!acq_bwd_shape_ok(fidelity, d, M, S, n)) return 0;
+  return acq_bwd_layout(fidelity, d, M, S, n).total;
+}
+
+int mobo_acq_moments_bwd(int fidelity, int d, int M, int S, long long n, const double* Zx,
+                         const double* const* zf, const double* const* theta, const double* const* ops,
+                         const double* const* samples, const double* raw_noise, double noise_lower,
+                         double noise_upper, const double* X, const double* d_mu, const double* d_var,
+                         int accumulate, double* dX, double* d_raw_noise, double* work, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!acq_bwd_shape_ok(fidelity, d, M, S, n)) return -2;
+  const AcqBwdLayout y = acq_bwd_layout(fidelity, d, M, S, n);
+  double* w = work;
+  // 1. the forward of mobo_acq_moments, every layer's moments and t / u kept
+  RowArgs rows[kMaxLayers];
+  for (int l = 0; l <= fidelity; ++l) {
+    fill_acq_row_args(rows[l], l, d, M, S, n, Zx, zf, theta, ops, samples, X, l == 0 ? nullptr : w + y.mu[l - 1],
+                      l == 0 ? nullptr : w + y.var[l - 1]);
+    RowArgs a = rows[l];
+    a.mu = w + y.mu[l]; a.var = w + y.var[l]; a.Tsave = w + y.Ts[l]; a.Usave = w + y.Us[l];
+    MOBO_TRY(launch_row_fwd(a, st));
+  }
+  // 2. moment matching -> d mu, d var of the top layer's rows (and the partials of d / d raw_noise)
+  {
+    AcqMomentBwdArgs a;
+    a.n = n; a.S = S; a.tiled = fidelity >= 1 ? 1 : 0;
+    a.mu = w + y.mu[fidelity]; a.var = w + y.var[fidelity];
+    a.noise_lo = noise_lower; a.noise_hi = noise_upper; a.raw_noise = raw_noise;
+    a.d_mu = d_mu; a.d_var = d_var; a.dmu = w + y.dmu; a.dvar = w + y.dvar;
+    a.part = d_raw_noise ? w + y.noise_part : nullptr;
+    MOBO_LAUNCH("acq_moment_bwd_kernel", st,
+                acq_moment_bwd_kernel<<<y.noise_blocks, ACQ_THREADS, 0, st>>>(a));
+    if (d_raw_noise) MOBO_TRY(launch_reduce_partials(w + y.noise_part, y.noise_blocks, 1, 1, d_raw_noise, accumulate, st));
+  }
+  // 3. row backward of every layer (d / dx of its rows, d / df of its propagated input), and through the propagation
+  //    into the moments of the layer below
+  for (int l = fidelity; l >= 0; --l) {
+    RowArgs a = rows[l];
+    fill_row_bwd_args(a, w + y.dmu, w + y.dvar, nullptr, w + y.Ts[l], w + y.Us[l], 0, l == 0 ? nullptr : w + y.df,
+                      w + y.dxrow[l]);
+    a.dk = w + y.dk;
+    MOBO_TRY(launch_row_bwd(a, st));
+    if (l >= 1) {
+      const long long Rp = rows[l - 1].R;
+      MOBO_LAUNCH("acq_prop_bwd_kernel", st,
+                  acq_prop_bwd_kernel<<<(unsigned)((Rp + ACQ_THREADS - 1) / ACQ_THREADS), ACQ_THREADS, 0, st>>>(
+                      w + y.df, w + y.var[l - 1], samples[l], Rp, l == 1 ? S : 1, S, w + y.dmu, w + y.dvar));
+    }
+  }
+  // 4. d / dX
+  {
+    AcqDxFoldArgs a;
+    a.n = n; a.d = d; a.S = S; a.nl = fidelity + 1; a.dX = dX; a.accumulate = accumulate;
+    for (int l = 0; l < kMaxLayers; ++l) a.dxrow[l] = l <= fidelity ? w + y.dxrow[l] : nullptr;
+    MOBO_LAUNCH("acq_dx_fold_kernel", st,
+                acq_dx_fold_kernel<<<(unsigned)((n * d + ACQ_THREADS - 1) / ACQ_THREADS), ACQ_THREADS, 0, st>>>(a));
+  }
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

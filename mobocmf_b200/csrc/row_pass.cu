@@ -1685,9 +1685,12 @@ int row_grid(long long R) {
   return (int)(ntiles < cap ? (ntiles > 0 ? ntiles : 1) : cap);
 }
 
+// 32-bit row indices in the kernels; callers chunk (MFDGP.ACQ_CHUNK, MFDGP.ACQ_GRAD_CHUNK)
+constexpr long long kMaxRows = (1ll << 31) - TR;
+
 int launch_row_fwd(const RowArgs& a, cudaStream_t st) {
   if (a.MP % 32 != 0 || a.MP > MAX_MP || a.d > kMaxD || a.M > a.MP) return -2;
-  if (a.R >= (1ll << 31) - TR) return -2;      // 32-bit row indices in the kernel; callers chunk (MFDGP.ACQ_CHUNK)
+  if (a.R >= kMaxRows) return -2;
   const size_t smem = row_smem_bytes(a.MP);
   static bool attr_done[kMaxDevices] = {false};
   if (first_on_device(attr_done))

@@ -273,6 +273,100 @@ __global__ void moment_kernel(const __grid_constant__ MomentArgs a) {
   a.out_var[i] = s2 / (double)a.S - mean * mean;
 }
 
+// ---- backward of the acquisition chain (mobo_acq_moments_bwd) ---------------------------------------------------
+// moment matching, per candidate i (tiled: rows i*S+s; untiled, fidelity 0: the S copies of row i coincide):
+//   dmu_s = d_mu / S + d_var 2 (mu_s - out_mu) / S,   dv_s = d_var / S [v_s + noise >= 1e-10]
+//   untiled: dmu = d_mu, dv = d_var [v + noise >= 1e-10]
+// and, when `part` is set, the per-block partials of d / d raw_noise:
+//   sum_i d_var[i] (1/S) sum_s [v_s + noise >= 1e-10] (hi - lo) sigmoid'(raw)
+// (folded in a fixed order by reduce_partials_kernel).  d_mu / d_var NULL: zero.
+struct AcqMomentBwdArgs {
+  long long n; int S; int tiled;
+  const double* mu; const double* var; double noise_lo, noise_hi; const double* raw_noise;
+  const double* d_mu; const double* d_var;
+  double* dmu; double* dvar;  // [R] of the top layer
+  double* part;               // [gridDim.x] or NULL
+};
+constexpr int ACQ_THREADS = 256;
+__global__ void __launch_bounds__(ACQ_THREADS) acq_moment_bwd_kernel(const __grid_constant__ AcqMomentBwdArgs a) {
+  __shared__ double red[ACQ_THREADS / 32];
+  const long long i = (long long)blockIdx.x * ACQ_THREADS + threadIdx.x;
+  const double sg = sigmoid_fwd(*a.raw_noise);
+  const double noise = a.noise_lo + (a.noise_hi - a.noise_lo) * sg;
+  double dn = 0.0;
+  if (i < a.n) {
+    const double gm = a.d_mu ? a.d_mu[i] : 0.0, gv = a.d_var ? a.d_var[i] : 0.0;
+    if (a.tiled) {
+      double s1 = 0.0;      // out_mu exactly as moment_kernel sums it
+      for (int s = 0; s < a.S; ++s) s1 += a.mu[i * a.S + s];
+      const double mean = s1 / (double)a.S, inv = 1.0 / (double)a.S;
+      int live = 0;
+      for (int s = 0; s < a.S; ++s) {
+        const long long r = i * a.S + s;
+        const bool ok = a.var[r] + noise >= kMinVariance;
+        a.dmu[r] = gm * inv + gv * 2.0 * (a.mu[r] - mean) * inv;
+        a.dvar[r] = ok ? gv * inv : 0.0;
+        live += ok;
+      }
+      dn = gv * (double)live / (double)a.S;
+    } else {
+      const bool ok = a.var[i] + noise >= kMinVariance;
+      a.dmu[i] = gm;
+      a.dvar[i] = ok ? gv : 0.0;
+      dn = ok ? gv : 0.0;
+    }
+  }
+  if (!a.part) return;
+  dn = warp_sum(dn);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = dn;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < ACQ_THREADS / 32; ++w) s += red[w];
+    a.part[blockIdx.x] = s * (a.noise_hi - a.noise_lo) * sg * (1.0 - sg);
+  }
+}
+
+// through the sample propagation f = mu_prev + sqrt(max(var_prev, 1e-10)) eps of the layer above, per row i of the
+// layer below (the rows i*prep .. i*prep+prep-1 above read it, row r reads eps[r % S]):
+//   dmu_prev[i] = sum_s df[i*prep+s],   dvar_prev[i] = [var_prev >= 1e-10] sum_s df eps / (2 sqrt(max(var_prev, 1e-10)))
+__global__ void __launch_bounds__(ACQ_THREADS) acq_prop_bwd_kernel(const double* __restrict__ df,
+                                                                   const double* __restrict__ var_prev,
+                                                                   const double* __restrict__ eps, long long R_prev,
+                                                                   int prep, int S, double* __restrict__ dmu_prev,
+                                                                   double* __restrict__ dvar_prev) {
+  const long long i = (long long)blockIdx.x * ACQ_THREADS + threadIdx.x;
+  if (i >= R_prev) return;
+  const long long base = i * prep;
+  double s0 = 0.0, s1 = 0.0;
+  for (int s = 0; s < prep; ++s) {
+    const double g = df[base + s];
+    s0 += g;
+    s1 = fma(g, eps[(base + s) % S], s1);
+  }
+  const double v = var_prev[i];
+  dmu_prev[i] = s0;
+  dvar_prev[i] = v >= kMinVariance ? s1 / (2.0 * sqrt(v)) : 0.0;
+}
+
+// dX[i][c] (+)= sum_l sum_{s < xrep_l} dxrow_l[i*xrep_l+s][c]: layer 0 first (xrep 1), then the layers above
+// (xrep S), s ascending
+struct AcqDxFoldArgs {
+  long long n; int d, S, nl;
+  const double* dxrow[kMaxLayers];
+  double* dX; int accumulate;
+};
+__global__ void __launch_bounds__(ACQ_THREADS) acq_dx_fold_kernel(const __grid_constant__ AcqDxFoldArgs a) {
+  const long long k = (long long)blockIdx.x * ACQ_THREADS + threadIdx.x;
+  if (k >= a.n * a.d) return;
+  const long long i = k / a.d;
+  const int c = (int)(k - i * a.d);
+  double s = a.dxrow[0][k];
+  for (int l = 1; l < a.nl; ++l)
+    for (int j = 0; j < a.S; ++j) s += a.dxrow[l][(i * a.S + j) * a.d + c];
+  a.dX[k] = a.accumulate ? a.dX[k] + s : s;
+}
+
 __global__ void jes_kernel(const double* __restrict__ vu, const double* __restrict__ vc, double* __restrict__ out,
                            long long n, int accumulate) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

@@ -1,6 +1,8 @@
 """torch.autograd wrappers over the C-ABI kernels: one Function for the per-step M x M operator chain of a layer
 (``layer_operators``) and one for the fused row pass (``layer_rows``).  They compose under torch autograd, so the
-ELBO step, the conditioned step and d acquisition / d X for ``optimize_acqf`` all run through the same kernels.
+ELBO step, the conditioned step and the acquisition of the models the fused chain does not serve all run through the
+same kernels.  ``acq_moments`` is the fused acquisition chain of one model, whose backward (d / dX for
+``optimize_acqf``) is one C-ABI call per chunk of candidates.
 
 Reference code replaced: UnwhitenedVariationalStrategy.forward / kl_mvn_mvn [upstream gpytorch] as reached from
 ``mobocmf/layers/mfdgp_hidden_layer.py:232-286,542-559`` and ``mobocmf/mlls/variational_elbo_mf.py:40``.
@@ -188,3 +190,81 @@ def layer_rows(ops, theta, zf, Zx, x, mu_prev=None, var_prev=None, eps=None, f_d
         eps_mod = eps.numel() if eps is not None else 1
     return _LayerRows.apply(ops, theta, zf, Zx, x, mu_prev, var_prev, eps, f_direct, kind, xrep, prep, eps_mod, R,
                             training)
+
+
+class AcqChain(object):
+    """The constants of one model's eval-mode acquisition chain up to layer ``fidelity``: per layer the operator
+    buffer, constrained theta, propagated inducing column zf and S fixed normals (None at layer 0), the shared
+    inducing inputs Zx and the likelihood's noise bounds."""
+
+    def __init__(self, fidelity, M, S, Zx, zf, theta, ops, samples, noise_lower, noise_upper):
+        self.fidelity, self.M, self.S, self.Zx = fidelity, M, S, Zx
+        self.zf, self.theta, self.ops, self.samples = zf, theta, ops, samples
+        self.noise_lower, self.noise_upper = noise_lower, noise_upper
+
+
+def _acq_forward(chain, X, raw_noise, chunk):
+    lib = _lib.load()
+    c = chain
+    n, d = X.shape
+    out_mu = torch.empty(n, dtype=torch.float64, device=X.device)
+    out_var = torch.empty(n, dtype=torch.float64, device=X.device)
+    chunk = min(n, chunk)
+    scratch = torch.empty(4 * chunk * c.S, dtype=torch.float64, device=X.device)
+    for a in range(0, n, chunk):
+        b = min(n, a + chunk)
+        _lib.check(lib.mobo_acq_moments(c.fidelity, d, c.M, c.S, b - a, _lib.ptr(c.Zx), _lib.ptr_array(c.zf),
+                                        _lib.ptr_array(c.theta), _lib.ptr_array(c.ops), _lib.ptr_array(c.samples),
+                                        _lib.ptr(raw_noise), c.noise_lower, c.noise_upper, _lib.ptr(X[a:b]),
+                                        _lib.ptr(out_mu[a:b]), _lib.ptr(out_var[a:b]), _lib.ptr(scratch),
+                                        _lib.stream_ptr()), "mobo_acq_moments")
+    return out_mu, out_var
+
+
+class _AcqMoments(torch.autograd.Function):
+    """(out_mu, out_var) of the acquisition chain, differentiable with respect to X and raw_noise.  The forward keeps
+    no rows: the backward recomputes each chunk's forward (mobo_acq_moments_bwd), so the memory of d / dX is bounded
+    by the chunk, not by the number of candidates."""
+
+    @staticmethod
+    def forward(ctx, X, raw_noise, chain, chunk, grad_chunk):
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(X, raw_noise)
+        ctx.chain, ctx.grad_chunk = chain, grad_chunk
+        return _acq_forward(chain, _c(X), _c(raw_noise), chunk)
+
+    @staticmethod
+    def backward(ctx, d_mu, d_var):
+        lib = _lib.load()
+        X, raw_noise = ctx.saved_tensors
+        c = ctx.chain
+        X, rn = _c(X), _c(raw_noise)
+        d_mu, d_var = _c(d_mu), _c(d_var)
+        n, d = X.shape
+        dX = torch.zeros(n, d, dtype=torch.float64, device=X.device)
+        dn = torch.zeros(1, dtype=torch.float64, device=X.device) if ctx.needs_input_grad[1] else None
+        chunk = min(n, ctx.grad_chunk)
+        work = torch.empty(lib.mobo_acq_bwd_work_doubles(c.fidelity, d, c.M, c.S, chunk), dtype=torch.float64,
+                           device=X.device)
+        # chunks write disjoint rows of dX; d raw_noise sums over all of them
+        for a in range(0, n, chunk):
+            b = min(n, a + chunk)
+            _lib.check(lib.mobo_acq_moments_bwd(
+                c.fidelity, d, c.M, c.S, b - a, _lib.ptr(c.Zx), _lib.ptr_array(c.zf), _lib.ptr_array(c.theta),
+                _lib.ptr_array(c.ops), _lib.ptr_array(c.samples), _lib.ptr(rn), c.noise_lower, c.noise_upper,
+                _lib.ptr(X[a:b]), None if d_mu is None else _lib.ptr(d_mu[a:b]),
+                None if d_var is None else _lib.ptr(d_var[a:b]), 1, _lib.ptr(dX[a:b]), _lib.ptr(dn), _lib.ptr(work),
+                _lib.stream_ptr()), "mobo_acq_moments_bwd")
+        return (dX if ctx.needs_input_grad[0] else None, None if dn is None else dn.reshape(raw_noise.shape),
+                None, None, None)
+
+
+def acq_moments(chain, X, raw_noise, chunk, grad_chunk):
+    """Moment-matched (mean, variance) over the S samples of the acquisition chain for the n candidates X (n, d):
+    MFDGP.predict_for_acquisition (models/mfdgp.py:237-262) in enqueues of ``chunk`` candidates.  When X requires a
+    gradient, the result is differentiable with respect to X and raw_noise, and the backward runs in chunks of
+    ``grad_chunk`` candidates."""
+    if torch.is_grad_enabled() and X.requires_grad:
+        return _AcqMoments.apply(X, raw_noise, chain, chunk, grad_chunk)
+    with torch.no_grad():
+        return _acq_forward(chain, X, raw_noise, chunk)

@@ -247,8 +247,14 @@ class MFDGP(nn.Module):
         second_moment = torch.mean(vars_tilde + mus_tilde ** 2, 1)
         return mus, second_moment - mus ** 2
 
-    # ---- fused acquisition chain (mobo_acq_moments): no autograd graph, one enqueue per model ----
+    # ---- fused acquisition chain (mobo_acq_moments, backward mobo_acq_moments_bwd): one enqueue per model and chunk ----
     ACQ_CHUNK = 1 << 18      # candidates per enqueue (bounds the n * S scratch)
+    # candidates per backward enqueue.  The backward recomputes the chunk's forward and keeps t and u of every row of
+    # every layer: about (2 MP + 2 + d)(1 + fidelity S) + (MP + 3) S doubles per candidate, 264 KB at M = 256, S = 25,
+    # fidelity 2 (C5), so 4096 candidates take 1.08 GB of work, whatever the total n (more layers take more per
+    # candidate).  A multiple of 32, so that every chunk starts its rows on the same tile and warp-group boundaries as
+    # one unchunked call: dX does not depend on the chunking.
+    ACQ_GRAD_CHUNK = 4096
 
     def clip_inducing_values(self, x_0, x_1, y_1):
         """y_1 at the point of x_1 nearest to each row of x_0 (models/mfdgp.py:125-135)."""
@@ -274,8 +280,6 @@ class MFDGP(nn.Module):
     def _fused_acquisition_applies(self, x):
         if self.training or self.use_only_highest_fidelity is True or not x.is_cuda or x.dtype != torch.float64:
             return False
-        if torch.is_grad_enabled() and x.requires_grad:
-            return False                       # d acquisition / dX goes through the composable autograd path
         layers = [getattr(self, self.name_hidden_layer + str(i)) for i in range(self.num_hidden_layers)]
         for lay in layers[1:]:
             lay._propagated_inducing_column()
@@ -284,10 +288,7 @@ class MFDGP(nn.Module):
         return True
 
     def _predict_for_acquisition_fused(self, x, fidelity_layer):
-        from .. import _lib
-        lib = _lib.load()
-        S = self.num_samples_for_acquisition
-        n, d = x.shape
+        from .. import functional as F
         layers = [getattr(self, self.name_hidden_layer + str(i)) for i in range(fidelity_layer + 1)]
         with torch.no_grad():
             trip = [lay.operators() for lay in layers]
@@ -296,25 +297,16 @@ class MFDGP(nn.Module):
             zf = [None if t[2] is None else t[2].detach().contiguous() for t in trip]
             smp = [None] + [lay._samples_on(x.device) for lay in layers[1:]]
             lik = getattr(self, self.name_hidden_layer_likelihood + str(fidelity_layer))
-            rn = lik.noise_covar.raw_noise
             c = lik.noise_covar.raw_noise_constraint
             key = ("noise_bounds", fidelity_layer)
             if key not in layers[0]._dev_cache:
                 layers[0]._dev_cache[key] = (float(c.lower_bound), float(c.upper_bound))
             lo, hi = layers[0]._dev_cache[key]
-            out_mu = torch.empty(n, dtype=torch.float64, device=x.device)
-            out_var = torch.empty(n, dtype=torch.float64, device=x.device)
-            chunk = min(n, self.ACQ_CHUNK)
-            scratch = torch.empty(4 * chunk * S, dtype=torch.float64, device=x.device)
-            M = layers[0].num_inducing
-            for a in range(0, n, chunk):
-                b = min(n, a + chunk)
-                _lib.check(lib.mobo_acq_moments(fidelity_layer, d, M, S, b - a, _lib.ptr(layers[0]._Zx()),
-                                                _lib.ptr_array(zf), _lib.ptr_array(theta), _lib.ptr_array(ops),
-                                                _lib.ptr_array(smp), _lib.ptr(rn), lo, hi, _lib.ptr(x[a:b]),
-                                                _lib.ptr(out_mu[a:b]), _lib.ptr(out_var[a:b]), _lib.ptr(scratch),
-                                                _lib.stream_ptr()), "mobo_acq_moments")
-        return out_mu, out_var
+        chain = F.AcqChain(fidelity_layer, layers[0].num_inducing, self.num_samples_for_acquisition, layers[0]._Zx(),
+                           zf, theta, ops, smp, lo, hi)
+        # with X.requires_grad, differentiable with respect to X and the likelihood's raw_noise (the one parameter the
+        # eval-mode chain does not hold constant, as on the composable path)
+        return F.acq_moments(chain, x, lik.noise_covar.raw_noise, self.ACQ_CHUNK, self.ACQ_GRAD_CHUNK)
 
     def find_good_initial_inducing_points_and_values(self, x_train, y_train, fidelities, layer):
         """models/mfdgp.py:290-317, vectorised: nearest same-fidelity neighbour by the reference's expansion
