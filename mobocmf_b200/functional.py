@@ -26,8 +26,9 @@ def ops_layout(M):
     MP = padded_m(M)
     MP2 = MP * MP
     return {"MP": MP, "L": 0, "W": MP2, "WT": 2 * MP2, "H": 3 * MP2, "HT": 4 * MP2, "P": 5 * MP2, "LQ": 6 * MP2,
-            "beta": 11 * MP2, "alpha": 11 * MP2 + MP, "scal": 11 * MP2 + 2 * MP, "flags": 11 * MP2 + 6 * MP + 16,
-            "size": 11 * MP2 + 6 * MP + 16 + 128}
+            "WF": 7 * MP2, "HTF": 8 * MP2, "HF": 9 * MP2, "WTF": 10 * MP2,
+            "beta": 11 * MP2, "alpha": 11 * MP2 + MP, "scal": 11 * MP2 + 2 * MP, "rowstat": 11 * MP2 + 2 * MP + 16,
+            "flags": 11 * MP2 + 6 * MP + 16, "size": 11 * MP2 + 6 * MP + 16 + 128}
 
 
 def _c(t):
