@@ -160,6 +160,19 @@ int mobo_step_ctx_wait_layer(void* ctx, int layer, void* stream);
 void mobo_step_side_stream(int on);
 int mobo_elbo_step(const mobo_step_desc* desc, void* stream);
 
+/* ELBO steps of the K black-box models of a BO iteration at the reference's sizes (M <= 64) in one launch: one CTA
+ * runs one model's complete step, the work of mobo_elbo_step (BlackBoxMFDGPFitter._update_model,
+ * mobocmf/util/blackbox_mfdgp_fitter.py:156-173, for every model that _train_mfdgp trains).  descs[i] has exactly
+ * mobo_elbo_step's meaning (out[8], accumulate, NULL gradient = frozen, g_Lq lower triangle with zeros above), except
+ * that desc.ctx is ignored: there is no side stream, and mobo_step_ctx_wait_layer does not apply.  desc.workspace:
+ * mobo_elbo_step_small_workspace_doubles(...) doubles (not mobo_elbo_step's size).  Preconditions: those of
+ * mobo_elbo_step, and M <= 64.  Returns -2 before any launch when n_models < 1 or any descriptor has M outside
+ * [1, 64], d outside [1, 8], L outside [1, 8] or B < 1 (the workspace query returns 0 for those).  Up to 8 models go
+ * into one launch of small_step_kernel; more models mean more launches.  Each model's result is independent of the
+ * others in the launch (fixed summation orders, no atomics).  CUDA-graph capturable. */
+size_t mobo_elbo_step_small_workspace_doubles(int L, int d, int M, int S, long long B);
+int mobo_elbo_step_small(const mobo_step_desc* descs, int n_models, void* stream);
+
 /* torch.optim.Adam update (mobocmf/util/blackbox_mfdgp_fitter.py:126,132,259; defaults betas (0.9, 0.999),
  * eps 1e-8, no weight decay) of nt <= 64 tensors in one launch.  step = 1-based step count after increment, or, for
  * CUDA-graph replays, step_dev != NULL: a device-resident count (advance it with mobo_adam_tick before each update;

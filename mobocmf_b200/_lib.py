@@ -38,6 +38,8 @@ _SIGNATURES = {
     # fused step / optimiser / acquisition chain (struct pointers travel as void*; see mobocmf_b200/fused.py)
     "mobo_elbo_step_workspace_doubles": (_c_sz, [_c_i, _c_i, _c_i, _c_i, _c_ll]),
     "mobo_elbo_step": (_c_i, [_c_dp, _c_dp]),
+    "mobo_elbo_step_small_workspace_doubles": (_c_sz, [_c_i, _c_i, _c_i, _c_i, _c_ll]),
+    "mobo_elbo_step_small": (_c_i, [_c_dp, _c_i, _c_dp]),
     "mobo_step_side_stream": (None, [_c_i]),
     "mobo_step_ctx_create": (_c_dp, []),
     "mobo_step_ctx_destroy": (None, [_c_dp]),

@@ -7,6 +7,7 @@
 #include "opchain.cu"
 #include "row_pass.cu"
 #include "step.cu"
+#include "small_step.cu"
 #include "rff.cu"
 
 using namespace mobo;
@@ -505,6 +506,40 @@ int mobo_elbo_step(const mobo_step_desc* D, void* stream) {
                     add_matrix_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(D->layer[l].g_Lq, dLq[l], n));
       }
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+static bool small_shape_ok(int L, int d, int M, long long B) {
+  return L >= 1 && L <= kMaxLayers && d >= 1 && d <= kMaxD && M >= 1 && M <= SS_MAX_M && B >= 1;
+}
+
+size_t mobo_elbo_step_small_workspace_doubles(int L, int d, int M, int S, long long B) {
+  if (!small_shape_ok(L, d, M, B)) return 0;
+  return ss_workspace_doubles(L, M, S < 1 ? 1 : S, B);
+}
+
+// SS_PER_LAUNCH descriptors per launch (they travel as the kernel's parameter, no host-to-device copy), one CTA each
+int mobo_elbo_step_small(const mobo_step_desc* descs, int n_models, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n_models < 1 || !descs) return -2;
+  for (int i = 0; i < n_models; ++i)
+    if (!small_shape_ok(descs[i].L, descs[i].d, descs[i].M, descs[i].B)) return -2;
+  static bool attr_done[kMaxDevices] = {false};
+  if (first_on_device(attr_done))
+    cudaFuncSetAttribute(small_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)ss_smem_bytes(SS_MAX_M));
+  for (int i0 = 0; i0 < n_models; i0 += SS_PER_LAUNCH) {
+    SmallBatch b;
+    memset(&b, 0, sizeof(b));
+    b.n = n_models - i0 < SS_PER_LAUNCH ? n_models - i0 : SS_PER_LAUNCH;
+    int maxM = 1;
+    for (int i = 0; i < b.n; ++i) {
+      b.desc[i] = descs[i0 + i];
+      if (b.desc[i].M > maxM) maxM = b.desc[i].M;
+    }
+    MOBO_LAUNCH("small_step_kernel", st, small_step_kernel<<<b.n, SS_THREADS, ss_smem_bytes(maxM), st>>>(b));
+    if (cudaGetLastError() != cudaSuccess) return -1;
+  }
+  return 0;
 }
 
 int mobo_adam(int nt, const mobo_adam_tensor* tensors, double lr, double beta1, double beta2, double eps,

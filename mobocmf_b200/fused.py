@@ -195,17 +195,20 @@ class FusedELBOStep(object):
 
     MAX_UNPINNED_WORKSPACES = 2
 
-    def _workspace(self, B, S, pin=False):
+    def _workspace(self, B, S, pin=False, small=False):
         """Scratch of the step for a (B, S) shape.  A captured CUDA graph bakes the workspace's address in, so a
         workspace that a graph references (``pin=True``) lives as long as this object; the others are kept for the
-        last few shapes only (full batch + ragged last batch of an epoch)."""
-        key = (B, S)
+        last few shapes only (full batch + ragged last batch of an epoch).  ``small``: the scratch of
+        ``mobo_elbo_step_small`` (its own size query) instead of ``mobo_elbo_step``'s."""
+        key = (B, S, "small") if small else (B, S)
         ws = self._ws.get(key)
         if ws is None:
             loose = [k for k in self._ws if k not in self._ws_pinned]
             while len(loose) >= self.MAX_UNPINNED_WORKSPACES:
                 del self._ws[loose.pop(0)]
-            n = self.lib.mobo_elbo_step_workspace_doubles(self.L, self.d, self.M, S, B)
+            query = self.lib.mobo_elbo_step_small_workspace_doubles if small else \
+                self.lib.mobo_elbo_step_workspace_doubles
+            n = query(self.L, self.d, self.M, S, B)
             ws = torch.empty(n, dtype=torch.float64, device=self.device)
             self._ws[key] = ws
         else:
@@ -234,6 +237,15 @@ class FusedELBOStep(object):
         """Returns (loss = -ELBO, KL * B / N) as 0-d device tensors (views of one result buffer, overwritten by the
         next call) and writes the gradients.  ``eps``: optional list indexed by layer of the training normals
         (B*S values for layers >= 1; reference: float32 ``torch.normal`` of shape (1, B), quirk Q6)."""
+        keep = self._stage(x_batch, y_batch, fidelities, eps, num_samples, accumulate, check_shortcut,
+                           pin_workspace, small=False)
+        _lib.check(self.lib.mobo_elbo_step(ctypes.byref(self._desc), _lib.stream_ptr()), "mobo_elbo_step")
+        return self._launched(keep)
+
+    def _stage(self, x_batch, y_batch, fidelities, eps, num_samples, accumulate, check_shortcut, pin_workspace,
+               small):
+        """Fills ``self._desc`` for one step on this minibatch (the launch is the caller's); returns the tensors the
+        enqueued step reads, which must stay alive until the next call."""
         B = x_batch.shape[0]
         S = int(num_samples)
         if x_batch.shape[1] != self.d or y_batch.numel() != B or fidelities.numel() != B:
@@ -260,9 +272,11 @@ class FusedELBOStep(object):
         D.layer[0].eps = None
         D.S, D.B, D.num_data = S, B, int(self.elbo.num_data)
         D.x, D.y, D.fid = x.data_ptr(), y.data_ptr(), f.data_ptr()
-        D.workspace = self._workspace(B, S, pin=pin_workspace).data_ptr()
+        D.workspace = self._workspace(B, S, pin=pin_workspace, small=small).data_ptr()
         D.accumulate = 1 if accumulate else 0
-        _lib.check(self.lib.mobo_elbo_step(ctypes.byref(D), _lib.stream_ptr()), "mobo_elbo_step")
+        return keep
+
+    def _launched(self, keep):
         self._last_inputs = keep          # keep the step's inputs alive until the next call (async kernels)
         for layer in self.layers:         # parameters are about to change: drop the composable path's cache
             layer._ops_cache = None
@@ -492,3 +506,145 @@ class GraphedELBOStep(object):
         for layer in self.step.layers:
             layer._ops_cache = None
         return self.loss, self.kl
+
+
+class SmallModelsELBOStep(object):
+    """The ELBO steps of several independent small MFDGPs (M <= 64: the reference's own problems) in ONE launch of
+    ``mobo_elbo_step_small``, one CTA per model: what ``BlackBoxMFDGPFitter._train_mfdgp`` does for the K black boxes
+    of a BO iteration (``mobocmf/util/blackbox_mfdgp_fitter.py:156-173`` per model), without the ~45 launches per
+    model-step of ``FusedELBOStep``.  Each model keeps its own ``FusedELBOStep`` (descriptor, flat gradient buffer,
+    ``out`` flags, ``check()``, the Q4 test ``applies()``); ``steps`` may pass existing ones to build on."""
+
+    MAX_M = 64
+
+    def __init__(self, models, elbos, steps=None):
+        ok, why = self.supported(models)
+        if not ok:
+            raise RuntimeError("small-model ELBO step not applicable: " + why)
+        self.steps = list(steps) if steps is not None else [FusedELBOStep(m, e) for m, e in zip(models, elbos)]
+        if len(self.steps) != len(models) or any(s.model is not m for s, m in zip(self.steps, models)):
+            raise ValueError("steps must be the FusedELBOStep of each model, in order")
+        self.lib = _bind()
+        self._descs = (StepDesc * len(self.steps))()
+
+    @staticmethod
+    def supported(models):
+        models = list(models)
+        if not models:
+            return False, "no models"
+        for m in models:
+            ok, why = FusedELBOStep.supported(m)
+            if not ok:
+                return False, why
+            if getattr(m, m.name_hidden_layer + "0").num_inducing > SmallModelsELBOStep.MAX_M:
+                return False, "more than %d inducing points" % SmallModelsELBOStep.MAX_M
+        return True, ""
+
+    def __call__(self, batches, eps=None, num_samples=1, accumulate=False, check_shortcut=True, pin_workspace=False):
+        """``batches[i] = (x, y, fid)`` of model i (each model its own B), or None: model i sits this step out.
+        ``eps[i]``: optional per-layer normals of model i, as ``FusedELBOStep``; ``num_samples``: one S for all models
+        or one per model.  Returns ``[(loss, kl)]`` per model (views of each model's result buffer; None for a model
+        that sat out)."""
+        if len(batches) != len(self.steps):
+            raise ValueError("one batch (or None) per model expected")
+        run, keeps = [], []
+        for i, (step, b) in enumerate(zip(self.steps, batches)):
+            if b is None:
+                continue
+            e = None if eps is None else eps[i]
+            S = num_samples[i] if isinstance(num_samples, (list, tuple)) else num_samples
+            keeps.append(step._stage(b[0], b[1], b[2], e, S, accumulate, check_shortcut, pin_workspace, small=True))
+            self._descs[len(run)] = step._desc
+            run.append(step)
+        if run:
+            _lib.check(self.lib.mobo_elbo_step_small(self._descs, len(run), _lib.stream_ptr()),
+                       "mobo_elbo_step_small")
+        res = {id(s): s._launched(k) for s, k in zip(run, keeps)}
+        return [res.get(id(s)) for s in self.steps]
+
+
+class GraphedSmallModelsELBOStep(object):
+    """``SmallModelsELBOStep`` plus every model's own ``Adam`` update captured in one CUDA graph per combination of
+    minibatch shapes (a ragged last batch gets its own graph) and replayed per step: one graph launch for all models.
+    Each optimiser reads its own model's ``out[6]`` as skip flag, so a model whose step failed skips only its own
+    update.  ``optimizers[i]`` must be ``Adam(..., capturable=True)`` over model i's parameters.  The training normals
+    are drawn inside the graph unless ``static_eps`` (the caller passes them on every call)."""
+
+    def __init__(self, small, optimizers, num_samples=1, warmup=3, static_eps=False):
+        if len(optimizers) != len(small.steps):
+            raise ValueError("one optimiser per model expected")
+        for o in optimizers:
+            if not isinstance(o, Adam) or not o.capturable:
+                raise ValueError("GraphedSmallModelsELBOStep needs mobocmf_b200.fused.Adam(capturable=True)")
+        self.small, self.optimizers, self.S = small, list(optimizers), int(num_samples)
+        for o, st in zip(self.optimizers, small.steps):
+            o.skip_flag = st.skip_flag
+        self.static_eps, self._warmup = static_eps, warmup
+        self.graphs = {}     # (batch shape or None per model) -> (static batches, static normals, graph, results)
+
+    def _run(self, static, static_eps):
+        res = self.small(static, eps=static_eps, num_samples=self.S, check_shortcut=False, pin_workspace=True)
+        for o, b in zip(self.optimizers, static):
+            if b is not None:
+                o.step()
+        return res
+
+    def _capture(self, batches, eps):
+        dev = self.small.steps[0].device
+        static, static_eps = [], None if not self.static_eps else []
+        for i, (st, b) in enumerate(zip(self.small.steps, batches)):
+            static.append(None if b is None else (b[0].detach().clone(), b[1].detach().clone().reshape(-1, 1),
+                                                  b[2].detach().clone().reshape(-1, 1)))
+            if self.static_eps:
+                B = 0 if b is None else b[0].shape[0]
+                static_eps.append([None] + [torch.zeros(B * self.S, dtype=torch.float64, device=dev)
+                                            for _ in range(1, st.L)])
+        # warm-up and capture run real updates: they must not count as training steps
+        snaps = [o.snapshot() for o in self.optimizers]
+        outs = [st.out.clone() for st in self.small.steps]
+        self._stage(static, static_eps, batches, eps)
+        s = torch.cuda.Stream()
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            for _ in range(self._warmup):
+                self._run(static, static_eps)
+        torch.cuda.current_stream().wait_stream(s)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            res = self._run(static, static_eps)
+        for o, snap in zip(self.optimizers, snaps):
+            o.restore(snap)
+        with torch.no_grad():
+            for st, o in zip(self.small.steps, outs):
+                st.out.copy_(o)      # sticky status flags: staging data of the warm-up steps does not count
+        return static, static_eps, graph, res
+
+    def _stage(self, static, static_eps, batches, eps):
+        for i, (dst, b) in enumerate(zip(static, batches)):
+            if dst is None:
+                continue
+            dst[0].copy_(b[0]); dst[1].copy_(b[1].reshape(-1, 1)); dst[2].copy_(b[2].reshape(-1, 1))
+            if static_eps is not None:
+                if eps is None:
+                    raise ValueError("this graph was built with static_eps=True: pass eps")
+                for l in range(1, self.small.steps[i].L):
+                    static_eps[i][l].copy_(eps[i][l].reshape(-1))
+
+    def __call__(self, batches, eps=None, check_shortcut=True):
+        """``batches[i] = (x, y, fid)`` of model i, or None (model i sits this step out: no step, no update).
+        Returns ``[(loss, kl)]`` per model (None for one that sat out)."""
+        if check_shortcut:
+            for st, b in zip(self.small.steps, batches):
+                if b is not None and not st.applies(b[0]):
+                    raise RuntimeError("x_batch equals the inducing inputs (quirk Q4 shortcut): use the composable "
+                                       "path for that model")
+        key = tuple(None if b is None else tuple(b[0].shape) for b in batches)
+        if key not in self.graphs:
+            self.graphs[key] = self._capture(batches, eps)
+        static, static_eps, graph, res = self.graphs[key]
+        self._stage(static, static_eps, batches, eps)
+        graph.replay()
+        for st in self.small.steps:
+            for layer in st.layers:
+                layer._ops_cache = None
+        return res

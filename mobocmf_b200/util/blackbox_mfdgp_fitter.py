@@ -335,6 +335,67 @@ class BlackBoxMFDGPFitter():
                 kl_iter += kl.detach()
         return loss_iter, kl_iter
 
+    # Where one CTA per model (mobo_elbo_step_small) beats one stream + graph per model (mobo_elbo_step), measured by
+    # tools/small_models_bench.py on an NVIDIA B200 at a 1000 W power limit (profiles/r03_small_models_bench.json,
+    # "sweep_S1"): for every group size K = 1, 3, 6 only up to M = 16 inducing points (at M = 24 it loses for K = 1, 3)
+    # and, at M = 16, up to 32 rows per model (at 64 rows it loses for K = 1, 3).
+    SMALL_STEP_MAX_INDUCING = 16
+    SMALL_STEP_MAX_ROWS = 32
+
+    def _small_group(self, hs, opts):
+        """The graphed single-kernel step of the models ``hs`` when it applies (SmallModelsELBOStep.supported: shared
+        inducing inputs, M <= 64) and pays (at most SMALL_STEP_MAX_INDUCING inducing points and SMALL_STEP_MAX_ROWS
+        rows per minibatch), and every model's loader yields the same number of batches per epoch (one replay per
+        batch index covers them all); else None."""
+        from ..fused import GraphedSmallModelsELBOStep, SmallModelsELBOStep
+        models = [h.mfdgp for h in hs]
+        ok, _ = SmallModelsELBOStep.supported(models)
+        if not ok:
+            return None
+        nbatches = {-(-h.num_data // h.train_loader.batch_size) for h in hs}
+        rows = max(min(h.num_data, h.train_loader.batch_size) for h in hs)
+        inducing = max(getattr(m, m.name_hidden_layer + "0").num_inducing for m in models)
+        if len(nbatches) != 1 or rows > self.SMALL_STEP_MAX_ROWS or inducing > self.SMALL_STEP_MAX_INDUCING:
+            return None
+        steps = [self._fused_step(h.mfdgp, h.elbo) for h in hs]
+        key = tuple(id(s) for s in steps)
+        cache = self.__dict__.setdefault("_small_steps", {})
+        if key not in cache:
+            cache[key] = SmallModelsELBOStep(models, [h.elbo for h in hs], steps=steps)
+        # the graph joins each member step's cache of the graphs it is replayed in (see _graphed_step), keyed by the
+        # group's optimisers: a new phase has new ones
+        okey = ("small",) + tuple(id(o) for o in opts)
+        graphs = steps[0].__dict__.setdefault("_graphs", {})
+        if okey not in graphs:
+            g = GraphedSmallModelsELBOStep(cache[key], opts)
+            for s in steps:
+                s.__dict__.setdefault("_graphs", {})[okey] = g
+        return graphs[okey]
+
+    @staticmethod
+    def _update_small_group(group, hs, opts):
+        """One epoch of every model of ``group``: per batch index one replay of the graphed small step.  A model whose
+        minibatch equals its inducing inputs (quirk Q4) takes ``_update_model``'s path for that batch."""
+        loss = [0.0] * len(hs)
+        kl = [0.0] * len(hs)
+        for batches in zip(*[h.train_loader for h in hs]):
+            active = [st.applies(b[0]) for st, b in zip(group.small.steps, batches)]
+            for n, (h, opt, b, a) in enumerate(zip(hs, opts, batches, active)):
+                if not a:
+                    l_n, k_n = BlackBoxMFDGPFitter._update_model(h.mfdgp, h.elbo, opt, [b])
+                    loss[n] += l_n
+                    kl[n] += k_n
+            if not any(active):
+                continue
+            for o, st in zip(opts, group.small.steps):
+                o.skip_flag = st.skip_flag
+            res = group([b if a else None for b, a in zip(batches, active)], check_shortcut=False)
+            for n, r in enumerate(res):
+                if r is not None:
+                    loss[n] += r[0].detach().clone()
+                    kl[n] += r[1].detach().clone()
+        return list(zip(loss, kl))
+
     def _train_mfdgp(self, func_update_model, fix_variational_hypers, num_epochs, lr):
         for kind, handlers in (("OBJ", self.mfdgp_handlers_objs), ("CON", self.mfdgp_handlers_cons)):
             opts = []
@@ -353,6 +414,16 @@ class BlackBoxMFDGPFitter():
                               loss_iter.item(), "\t KL per epoch:", kl_iter.item())
                         sys.stdout.flush()
 
+            group = None
+            if self.concurrent_models and self.use_cuda_graph and func_update_model == self._update_model:
+                group = self._small_group(hs, opts)
+            if group is not None:
+                # every model's step of one batch index in one graph replay (mobo_elbo_step_small + the K Adams)
+                for i in range(num_epochs):
+                    sums = self._update_small_group(group, hs, opts)
+                    for n, (loss_iter, kl_iter) in enumerate(sums):
+                        report(n, i, loss_iter, kl_iter)
+                continue
             if self.concurrent_models and len(hs) > 1:
                 cur = torch.cuda.current_stream(hs[0].device)
                 streams = [torch.cuda.Stream(device=h.device) for h in hs]
@@ -577,9 +648,12 @@ class BlackBoxMFDGPFitter():
         graphs = self.__dict__.pop("_cond_graphs", None)      # captured CUDA graphs / streams do not travel through
         self.__dict__.pop("_cond_streams", None)              # deepcopy
         self.__dict__.pop("_cond_substreams", None)
+        small = self.__dict__.pop("_small_steps", None)        # ctypes descriptors and graphs, like the elbos' steps
         self_copy = deepcopy(self)
         if graphs is not None:
             self._cond_graphs = graphs
+        if small is not None:
+            self._small_steps = small
         for h in handlers:
             h.mfdgp.train()
         for h in list(self_copy.mfdgp_handlers_objs.values()) + list(self_copy.mfdgp_handlers_cons.values()):
