@@ -125,4 +125,96 @@ __device__ __forceinline__ double kern_diag(const KernParams& kp, double f) {
   return kp.a1 * (kp.vlin * f * f + kp.af) + kp.a2;
 }
 
+// k((xa, fa), (xb, fb)) off the diagonal (fa, fb unused for kind 0)
+__device__ __forceinline__ double kern_entry(const KernParams& kp, int d, const double* xa, double fa, const double* xb,
+                                             double fb) {
+  double D1 = 0.0, D2 = 0.0;
+  for (int c = 0; c < d; ++c) {
+    const double df = xa[c] - xb[c];
+    D1 = fma(df * df, kp.il1[c], D1);
+    D2 = fma(df * df, kp.il2[c], D2);
+  }
+  const double E1 = exp(-0.5 * D1);
+  if (kp.kind == 0) return kp.a1 * E1;
+  const double dff = fa - fb;
+  return kp.a1 * E1 * (kp.vlin * fa * fb + kp.af * exp(-0.5 * dff * dff * kp.ilf)) + kp.a2 * exp(-0.5 * D2);
+}
+
+// accumulators of g * dk / dtheta: s[0..4] = d / d (a1, v, af, lf-term, a2), l1 / l2 = sum g (a1 E1 gg | a2 E2) D_c^2;
+// kern_theta_slot maps them to the theta layout
+struct KernAcc {
+  double s[5], l1[kMaxD], l2[kMaxD];
+  __device__ __forceinline__ void zero() {
+#pragma unroll
+    for (int q = 0; q < 5; ++q) s[q] = 0.0;
+#pragma unroll
+    for (int c = 0; c < kMaxD; ++c) { l1[c] = 0.0; l2[c] = 0.0; }
+  }
+};
+
+// g * dk((xa, fa), (xb, fb)) / dtheta into acc (off the diagonal); ca, cb = dk / dfa, dk / dfb WITHOUT the weight g
+// (0 for kind 0), so that each caller keeps its own accumulation order
+__device__ __forceinline__ void kern_entry_bwd(const KernParams& kp, int d, const double* xa, double fa,
+                                               const double* xb, double fb, double g, KernAcc& acc, double& ca,
+                                               double& cb) {
+  double d2[kMaxD], D1 = 0.0, D2 = 0.0;
+#pragma unroll
+  for (int c = 0; c < kMaxD; ++c) {
+    const double df = c < d ? xa[c] - xb[c] : 0.0;
+    d2[c] = df * df;
+    D1 = fma(d2[c], kp.il1[c], D1);
+    D2 = fma(d2[c], kp.il2[c], D2);
+  }
+  const double E1 = exp(-0.5 * D1);
+  if (kp.kind == 0) {
+    const double gkk = g * kp.a1 * E1;
+    acc.s[0] = fma(g, E1, acc.s[0]);
+#pragma unroll
+    for (int c = 0; c < kMaxD; ++c) acc.l1[c] = fma(gkk, d2[c], acc.l1[c]);
+    ca = 0.0; cb = 0.0;
+    return;
+  }
+  const double dff = fa - fb;
+  const double Ef = exp(-0.5 * dff * dff * kp.ilf), E2 = exp(-0.5 * D2);
+  const double gg = kp.vlin * fa * fb + kp.af * Ef;
+  const double s1 = kp.a1 * E1, s2 = kp.a2 * E2;
+  const double dEf = s1 * kp.af * Ef * dff * kp.ilf;
+  ca = s1 * kp.vlin * fb - dEf;
+  cb = s1 * kp.vlin * fa + dEf;
+  acc.s[0] = fma(g, E1 * gg, acc.s[0]);
+  acc.s[1] = fma(g, s1 * fa * fb, acc.s[1]);
+  acc.s[2] = fma(g, s1 * Ef, acc.s[2]);
+  acc.s[3] = fma(g, dEf * dff, acc.s[3]);
+  acc.s[4] = fma(g, E2, acc.s[4]);
+  const double g1 = g * s1 * gg, g2 = g * s2;
+#pragma unroll
+  for (int c = 0; c < kMaxD; ++c) { acc.l1[c] = fma(g1, d2[c], acc.l1[c]); acc.l2[c] = fma(g2, d2[c], acc.l2[c]); }
+}
+
+// g * d kern_diag(f) / dtheta into acc; returns g a1 v, so that g * d kern_diag / df = 2 (g a1 v) f (0 for kind 0)
+__device__ __forceinline__ double kern_diag_bwd(const KernParams& kp, double f, double g, KernAcc& acc) {
+  if (kp.kind == 0) { acc.s[0] += g; return 0.0; }
+  acc.s[0] += g * (kp.vlin * f * f + kp.af);
+  acc.s[1] += g * kp.a1 * f * f;
+  acc.s[2] += g * kp.a1;
+  acc.s[4] += g;
+  return g * kp.a1 * kp.vlin;
+}
+
+// accumulator q (s[0..4], then l1[0..kMaxD), then l2[0..kMaxD)) summed to s -> its theta slot (return value, -1:
+// none) and the value there: a length-scale sum times il^(3/2) is d / d l, s[3] (one il_f inside) times sqrt(il_f)
+__device__ __forceinline__ int kern_theta_slot(const KernParams& kp, int q, double s, double& out) {
+  if (q < 5) {
+    out = q == 3 ? s * sqrt(kp.ilf) : s;
+    return kp.kind == 1 ? q : (q == 0 ? 0 : -1);
+  }
+  const bool first = q < 5 + kMaxD;          // l1 (kind 0: its only length scales) or l2
+  const int c = first ? q - 5 : q - 5 - kMaxD;
+  const double il = first ? kp.il1[c] : kp.il2[c];
+  out = s * il * sqrt(il);
+  if (c >= kp.d) return -1;
+  if (kp.kind == 0) return first ? 1 + c : -1;
+  return first ? q : 5 + kp.d + c;
+}
+
 }  // namespace mobo

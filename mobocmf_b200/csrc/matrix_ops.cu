@@ -45,11 +45,8 @@ kzz_bwd_kernel(int kind, int d, int M, int MP, const double* Zx, const double* z
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int i = blockIdx.x * KZB_WARPS + warp;
-  double th_s[5], th_l1[kMaxD], th_l2[kMaxD];
-#pragma unroll
-  for (int q = 0; q < 5; ++q) th_s[q] = 0.0;
-#pragma unroll
-  for (int c = 0; c < kMaxD; ++c) { th_l1[c] = 0.0; th_l2[c] = 0.0; }
+  KernAcc acc;
+  acc.zero();
   double dzi = 0.0;
   if (i < M) {
     const double fi = kind == 1 ? zf[i] : 0.0;
@@ -59,64 +56,26 @@ kzz_bwd_kernel(int kind, int d, int M, int MP, const double* Zx, const double* z
     for (int j = lane; j < M; j += 32) {
       const double gk = dP[(size_t)i * MP + j];
       if (i == j) {
-        if (kind == 0) {
-          th_s[0] += gk;
-        } else {
-          th_s[0] += gk * (kp.vlin * fi * fi + kp.af);
-          th_s[1] += gk * kp.a1 * fi * fi;
-          th_s[2] += gk * kp.a1;
-          th_s[4] += gk;
-          dzi += gk * kp.a1 * kp.vlin * fi;     // doubled below -> 2 a1 v f
-        }
+        dzi += kern_diag_bwd(kp, fi, gk, acc) * fi;     // doubled below -> 2 a1 v f
         continue;
       }
-      double D1 = 0.0, D2 = 0.0, diff[kMaxD];
-#pragma unroll
-      for (int c = 0; c < kMaxD; ++c) {
-        diff[c] = c < d ? zi[c] - Zx[(size_t)j * d + c] : 0.0;
-        D1 = fma(diff[c] * diff[c], kp.il1[c], D1);
-        D2 = fma(diff[c] * diff[c], kp.il2[c], D2);
-      }
-      const double E1 = exp(-0.5 * D1);
-      if (kind == 0) {
-        const double gkk = gk * kp.a1 * E1;
-        th_s[0] = fma(gk, E1, th_s[0]);
-#pragma unroll
-        for (int c = 0; c < kMaxD; ++c) th_l1[c] = fma(gkk, diff[c] * diff[c], th_l1[c]);
-      } else {
-        const double fj = zf[j], dff = fi - fj;
-        const double Ef = exp(-0.5 * dff * dff * kp.ilf), E2 = exp(-0.5 * D2);
-        const double gg = kp.vlin * fi * fj + kp.af * Ef;
-        const double s1 = kp.a1 * E1, s2 = kp.a2 * E2;
-        const double dEf = s1 * kp.af * Ef * dff * kp.ilf;
-        dzi = fma(gk, s1 * kp.vlin * fj - dEf, dzi);
-        th_s[0] = fma(gk, E1 * gg, th_s[0]);
-        th_s[1] = fma(gk, s1 * fi * fj, th_s[1]);
-        th_s[2] = fma(gk, s1 * Ef, th_s[2]);
-        th_s[3] = fma(gk, dEf * dff, th_s[3]);
-        th_s[4] = fma(gk, E2, th_s[4]);
-        const double g1 = gk * s1 * gg, g2 = gk * s2;
-#pragma unroll
-        for (int c = 0; c < kMaxD; ++c) {
-          const double d2 = diff[c] * diff[c];
-          th_l1[c] = fma(g1, d2, th_l1[c]);
-          th_l2[c] = fma(g2, d2, th_l2[c]);
-        }
-      }
+      double ca, cb;
+      kern_entry_bwd(kp, d, zi, fi, Zx + (size_t)j * d, kind == 1 ? zf[j] : 0.0, gk, acc, ca, cb);
+      if (kind == 1) dzi = fma(gk, ca, dzi);
     }
   }
   dzi = warp_sum(dzi);
   if (lane == 0 && i < M && kind == 1 && dzf) dzf[i] = 2.0 * dzi;
 #pragma unroll
   for (int q = 0; q < 5; ++q) {
-    const double s = warp_sum(th_s[q]);
+    const double s = warp_sum(acc.s[q]);
     if (lane == 0) accw[warp][q] = s;
   }
 #pragma unroll
   for (int c = 0; c < kMaxD; ++c) {
-    double s = warp_sum(th_l1[c]);
+    double s = warp_sum(acc.l1[c]);
     if (lane == 0) accw[warp][5 + c] = s;
-    s = warp_sum(th_l2[c]);
+    s = warp_sum(acc.l2[c]);
     if (lane == 0) accw[warp][5 + kMaxD + c] = s;
   }
   __syncthreads();
@@ -124,20 +83,8 @@ kzz_bwd_kernel(int kind, int d, int M, int MP, const double* Zx, const double* z
   if (tid < kMaxTheta) {
     double s = 0.0;
     for (int w = 0; w < KZB_WARPS; ++w) s += accw[w][tid];
-    double out = 0.0;
-    int slot = -1;
-    if (kind == 0) {
-      if (tid == 0) { slot = 0; out = s; }
-      else if (tid >= 5 && tid < 5 + d) { slot = 1 + (tid - 5); out = s * kp.il1[tid - 5] * sqrt(kp.il1[tid - 5]); }
-    } else {
-      if (tid < 5) { slot = tid; out = tid == 3 ? s * sqrt(kp.ilf) : s; }
-      else if (tid < 5 + d) { slot = tid; out = s * kp.il1[tid - 5] * sqrt(kp.il1[tid - 5]); }
-      else if (tid >= 5 + kMaxD && tid < 5 + kMaxD + d) {
-        const int c = tid - 5 - kMaxD;
-        slot = 5 + d + c;
-        out = s * kp.il2[c] * sqrt(kp.il2[c]);
-      }
-    }
+    double out;
+    const int slot = kern_theta_slot(kp, tid, s, out);
     if (slot >= 0) part_theta[(size_t)blockIdx.x * kMaxTheta + slot] = out;
   }
 }

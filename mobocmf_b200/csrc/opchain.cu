@@ -152,16 +152,7 @@ __device__ inline double oc_kernel_entry(const KernParams& kp, int kind, int d, 
     }
     return v;
   }
-  double D1 = 0.0, D2 = 0.0;
-  for (int c = 0; c < d; ++c) {
-    const double df = Zx[(size_t)i * d + c] - Zx[(size_t)j * d + c];
-    D1 = fma(df * df, kp.il1[c], D1);
-    D2 = fma(df * df, kp.il2[c], D2);
-  }
-  const double E1 = exp(-0.5 * D1);
-  if (kind == 0) return kp.a1 * E1;
-  const double fi = zf[i], fj = zf[j], dff = fi - fj;
-  return kp.a1 * E1 * (kp.vlin * fi * fj + kp.af * exp(-0.5 * dff * dff * kp.ilf)) + kp.a2 * exp(-0.5 * D2);
+  return kern_entry(kp, d, Zx + (size_t)i * d, kind == 1 ? zf[i] : 0.0, Zx + (size_t)j * d, kind == 1 ? zf[j] : 0.0);
 }
 
 __global__ void __launch_bounds__(OC_THREADS) opchain_kernel(LayerBatch b, double jitter) {

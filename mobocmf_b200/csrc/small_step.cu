@@ -9,7 +9,9 @@
 //   ELBO terms (ell_kernel), row backward (dt, dk = W^T dt, through the covariance function), whitened statistics
 //   A2 / A1 / b, operator-chain backward (matrix_ops.cu), through K(Z, Z) (kzz_bwd_kernel), gradient assembly
 //   (step_finish_kernel).
-// The formulation is the one of those kernels; only the schedule differs.  M <= 64 keeps the six working M x M
+// The formulation is the one of those kernels, and so is the code of every per-entry and per-row formula: the
+// covariance entry and its derivatives (common.cuh), the constraint transforms, ELBO row term, propagation backward,
+// raw-gradient store and result flags (step.cu); only the schedule differs.  M <= 64 keeps the six working M x M
 // matrices of a layer in shared memory (6 x 33 KB at M = 64); per-row t = W k and u = H^T t go to the model's
 // workspace (L2-resident at these sizes).  Plain FP64 FMA: at M <= 64 a product is a few thousand FMAs per thread.
 // Every sum has a fixed order and there are no atomics: a model's result does not depend on the other models of the
@@ -64,79 +66,6 @@ __device__ inline SsLayer ss_layer(double* ws, size_t off, long long R, int M) {
   return y;
 }
 
-// k((xa, fa), (xb, fb)) off the diagonal, evaluated as oc_kernel_entry does
-__device__ __forceinline__ double ss_kern(const KernParams& kp, int d, const double* xa, double fa, const double* xb,
-                                          double fb) {
-  double D1 = 0.0, D2 = 0.0;
-  for (int c = 0; c < d; ++c) {
-    const double df = xa[c] - xb[c];
-    D1 = fma(df * df, kp.il1[c], D1);
-    D2 = fma(df * df, kp.il2[c], D2);
-  }
-  const double E1 = exp(-0.5 * D1);
-  if (kp.kind == 0) return kp.a1 * E1;
-  const double dff = fa - fb;
-  return kp.a1 * E1 * (kp.vlin * fa * fb + kp.af * exp(-0.5 * dff * dff * kp.ilf)) + kp.a2 * exp(-0.5 * D2);
-}
-
-// d theta accumulators in kzz_bwd_kernel's conventions: s[0..4] = scalars, l1 / l2 = sum g (a1 E1 gg | a2 E2) D_c^2
-struct SsAcc {
-  double s[5], l1[kMaxD], l2[kMaxD];
-  __device__ void zero() {
-#pragma unroll
-    for (int q = 0; q < 5; ++q) s[q] = 0.0;
-#pragma unroll
-    for (int c = 0; c < kMaxD; ++c) { l1[c] = 0.0; l2[c] = 0.0; }
-  }
-};
-
-// g * d k((xa, fa), (xb, fb)) / d theta into acc (off the diagonal); returns g dk/dfa and g dk/dfb
-__device__ __forceinline__ void ss_kern_bwd(const KernParams& kp, int d, const double* xa, double fa, const double* xb,
-                                            double fb, double g, SsAcc& acc, double& gfa, double& gfb) {
-  double d2[kMaxD], D1 = 0.0, D2 = 0.0;
-#pragma unroll
-  for (int c = 0; c < kMaxD; ++c) {
-    const double df = c < d ? xa[c] - xb[c] : 0.0;
-    d2[c] = df * df;
-    D1 = fma(d2[c], kp.il1[c], D1);
-    D2 = fma(d2[c], kp.il2[c], D2);
-  }
-  const double E1 = exp(-0.5 * D1);
-  if (kp.kind == 0) {
-    const double gkk = g * kp.a1 * E1;
-    acc.s[0] = fma(g, E1, acc.s[0]);
-#pragma unroll
-    for (int c = 0; c < kMaxD; ++c) acc.l1[c] = fma(gkk, d2[c], acc.l1[c]);
-    gfa = 0.0; gfb = 0.0;
-    return;
-  }
-  const double dff = fa - fb;
-  const double Ef = exp(-0.5 * dff * dff * kp.ilf), E2 = exp(-0.5 * D2);
-  const double gg = kp.vlin * fa * fb + kp.af * Ef;
-  const double s1 = kp.a1 * E1, s2 = kp.a2 * E2;
-  const double dEf = s1 * kp.af * Ef * dff * kp.ilf;
-  gfa = g * (s1 * kp.vlin * fb - dEf);
-  gfb = g * (s1 * kp.vlin * fa + dEf);
-  acc.s[0] = fma(g, E1 * gg, acc.s[0]);
-  acc.s[1] = fma(g, s1 * fa * fb, acc.s[1]);
-  acc.s[2] = fma(g, s1 * Ef, acc.s[2]);
-  acc.s[3] = fma(g, dEf * dff, acc.s[3]);
-  acc.s[4] = fma(g, E2, acc.s[4]);
-  const double g1 = g * s1 * gg, g2 = g * s2;
-#pragma unroll
-  for (int c = 0; c < kMaxD; ++c) { acc.l1[c] = fma(g1, d2[c], acc.l1[c]); acc.l2[c] = fma(g2, d2[c], acc.l2[c]); }
-}
-
-// g * d k_diag(fa) / d theta into acc; returns g dk_diag / dfa
-__device__ __forceinline__ double ss_diag_bwd(const KernParams& kp, double fa, double g, SsAcc& acc) {
-  if (kp.kind == 0) { acc.s[0] += g; return 0.0; }
-  acc.s[0] += g * (kp.vlin * fa * fa + kp.af);
-  acc.s[1] += g * kp.a1 * fa * fa;
-  acc.s[2] += g * kp.a1;
-  acc.s[4] += g;
-  return g * 2.0 * kp.a1 * kp.vlin * fa;
-}
-
 // sum over the CTA in a fixed order (butterfly within warps, then warps in order); every thread gets the result
 __device__ __forceinline__ double ss_block_sum(double v, double* red) {
   v = warp_sum(v);
@@ -150,8 +79,8 @@ __device__ __forceinline__ double ss_block_sum(double v, double* red) {
   return s;
 }
 
-// the CTA's SsAcc's -> d loss / d theta in the theta layout (kzz_bwd_kernel's final mapping), into out[kMaxTheta]
-__device__ void ss_reduce_acc(const SsAcc& acc, const KernParams& kp, int d, double (*red)[kMaxTheta], double* out) {
+// the CTA's accumulators -> d loss / d theta in the theta layout, into out[kMaxTheta]
+__device__ void ss_reduce_acc(const KernAcc& acc, const KernParams& kp, double (*red)[kMaxTheta], double* out) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, tid = threadIdx.x;
   double v[kMaxTheta];
 #pragma unroll
@@ -168,26 +97,12 @@ __device__ void ss_reduce_acc(const SsAcc& acc, const KernParams& kp, int d, dou
   if (tid < kMaxTheta) {
     double s = 0.0;
     for (int w = 0; w < SS_WARPS; ++w) s += red[w][tid];
-    int slot = -1;
-    double o = 0.0;
-    if (kp.kind == 0) {
-      if (tid == 0) { slot = 0; o = s; }
-      else if (tid >= 5 && tid < 5 + d) { slot = 1 + (tid - 5); o = s * kp.il1[tid - 5] * sqrt(kp.il1[tid - 5]); }
-    } else {
-      if (tid < 5) { slot = tid; o = tid == 3 ? s * sqrt(kp.ilf) : s; }
-      else if (tid < 5 + d) { slot = tid; o = s * kp.il1[tid - 5] * sqrt(kp.il1[tid - 5]); }
-      else if (tid >= 5 + kMaxD && tid < 5 + kMaxD + d) {
-        const int c = tid - 5 - kMaxD;
-        slot = 5 + d + c;
-        o = s * kp.il2[c] * sqrt(kp.il2[c]);
-      }
-    }
+    double o;
+    const int slot = kern_theta_slot(kp, tid, s, o);
     if (slot >= 0) out[slot] = o;
   }
   __syncthreads();
 }
-
-__device__ __forceinline__ void ss_store(double* dst, double g, int accumulate) { *dst = accumulate ? *dst + g : g; }
 
 // whitened statistics of a layer's rows: A2 = sum dvar t t^T -> mA2, A1 = the same over unclamped rows -> mA1 (both
 // full symmetric), b = sum dmu t -> vb.  Each thread owns up to 9 entries of the lower triangle, rows ascending; the
@@ -311,7 +226,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
     if (tid < nth) y.theta[tid] = softplus_fwd(*D.layer[l].raw_theta[tid]);
     if (tid == 32) {
       const mobo_layer_desc& ldsc = D.layer[l];
-      noise_s[l] = ldsc.noise_lower + (ldsc.noise_upper - ldsc.noise_lower) * sigmoid_fwd(*ldsc.raw_noise);
+      noise_s[l] = interval_fwd(ldsc.noise_lower, ldsc.noise_upper, *ldsc.raw_noise);
     }
   }
   __syncthreads();
@@ -429,7 +344,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
         const long long pr = r / prep;
         f = yp.mu[pr] + sqrt(fmax(yp.var[pr], kMinVariance)) * eps[r];
       }
-      for (int j = lane; j < M; j += 32) va[j] = ss_kern(kp, d, xr, f, Zx + (size_t)j * d, kind ? zf[j] : 0.0);
+      for (int j = lane; j < M; j += 32) va[j] = kern_entry(kp, d, xr, f, Zx + (size_t)j * d, kind ? zf[j] : 0.0);
       __syncwarp();
       double q1 = 0.0, mu = 0.0, q2 = 0.0;
       for (int i = lane; i < M; i += 32) {
@@ -478,26 +393,15 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
       double data = 0.0, ds2 = 0.0;
       for (long long r = tid; r < R; r += SS_THREADS) {
         const long long b = r / Sl;
-        const double w = (D.fid[b] == (double)l) ? 1.0 / (double)Sl : 0.0;
-        const double mu = y.mu[r], v = y.var[r];
-        const bool live = v >= kMinVariance;
-        const double vuu = live ? v : kMinVariance;
-        const double res = D.y[b] - mu;
-        const double q = res * res + vuu;
-        data += w * -0.5 * (q / s2 + log(s2) + kLog2Pi);
-        ds2 += w * 0.5 * (1.0 / s2 - q / (s2 * s2));
-        double dmu = -w * res / s2;
-        double dv = live ? w * 0.5 / s2 : 0.0;
+        const double v = y.var[r];
+        double ds2r, dmu, dv;
+        data += ell_row(D.y[b], D.fid[b], l, Sl, y.mu[r], v, s2, ds2r, dmu, dv);
+        ds2 += ds2r;
         if (has_next) {
-          double t0 = 0.0, t1 = 0.0;
-          const long long base = r * prep_next;
-          for (int k = 0; k < prep_next; ++k) {
-            const double g = df_next[base + k];
-            t0 += g;
-            t1 = fma(g, eps_next[base + k], t1);
-          }
-          dmu += t0;
-          if (live) dv += t1 / (2.0 * sqrt(vuu));
+          double gmu, gv;
+          prop_bwd(df_next, eps_next, r * prep_next, prep_next, 0, v, gmu, gv);
+          dmu += gmu;
+          dv += gv;
         }
         y.dmu[r] = dmu;
         y.dvar[r] = dv;
@@ -517,7 +421,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
     __syncthreads();
     // row backward: dt = dmu beta - 2 dvar (mask t - H u), dk = W^T dt, then through the covariance function
     {
-      SsAcc acc;
+      KernAcc acc;
       acc.zero();
       double az0 = 0.0, az1 = 0.0;
       for (long long r = warp; r < R; r += SS_WARPS) {
@@ -539,20 +443,22 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
           if (j >= M) break;
           double gk = 0.0;
           for (int i = j; i < M; ++i) gk = fma(mW[i * ld + j], va[i], gk);
-          double gfa, gfb;
-          ss_kern_bwd(kp, d, xr, f, Zx + (size_t)j * d, kind ? D.layer[l - 1].m[j] : 0.0, gk, acc, gfa, gfb);
+          double ca, cb;
+          kern_entry_bwd(kp, d, xr, f, Zx + (size_t)j * d, kind ? D.layer[l - 1].m[j] : 0.0, gk, acc, ca, cb);
+          // the weighted f-derivatives are rounded before they are summed (__dmul_rn: never fused into the sums)
+          const double gfa = __dmul_rn(gk, ca), gfb = __dmul_rn(gk, cb);
           gf += gfa;
           if (jj == 0) az0 += gfb; else az1 += gfb;
         }
         const double dvm = dvar * mask;
-        if (lane == 0) gf += ss_diag_bwd(kp, f, dvm, acc);
+        if (lane == 0) gf += __dmul_rn(2.0 * kern_diag_bwd(kp, f, dvm, acc), f);
         gf = warp_sum(gf);
         if (kind == 1 && lane == 0) y.df[r] = gf;
         __syncwarp();
       }
       if (lane < M) azf[warp][lane] = az0;
       if (lane + 32 < M) azf[warp][lane + 32] = az1;
-      ss_reduce_acc(acc, kp, d, red, th_rows);
+      ss_reduce_acc(acc, kp, red, th_rows);
     }
     // whitened statistics A2 = sum dvar t t^T -> mF, A1 = the same over unclamped rows -> mD, b = sum dmu t -> vb
     ss_stats(y.T, y.dvar, y.dmu, y.craw, R, M, ld, mC, mD, mF, vb, rowsc);
@@ -587,7 +493,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
       if (ldsc.g_m) {
         double g = s;
         if (l + 1 < L) g += dzr[j] + dzp[j];
-        ss_store(ldsc.g_m + j, g, D.accumulate);
+        store_grad(ldsc.g_m + j, g, D.accumulate);
       }
     }
     __syncthreads();
@@ -611,7 +517,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
           for (int k = i; k < M; ++k) v = fma(mW[k * ld + i], mC[k * ld + j], v);
           if (i == j) v -= kl_scale / lqd[i];
         }
-        ss_store(ldsc.g_Lq + idx, v, D.accumulate);
+        store_grad(ldsc.g_Lq + idx, v, D.accumulate);
       }
     }
     // dP = X1 W -> mF (A2 is no longer needed)
@@ -630,7 +536,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
     __syncthreads();
     // through K(Z, Z) (kzz_bwd_kernel): one warp per inducing point i, lanes over j
     {
-      SsAcc acc;
+      KernAcc acc;
       acc.zero();
       for (int i = warp; i < M; i += SS_WARPS) {
         const double* zf = kind ? D.layer[l - 1].m : nullptr;
@@ -639,29 +545,21 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
         for (int j = lane; j < M; j += 32) {
           const double gk = mF[i * ld + j];
           if (i == j) {
-            dzi += ss_diag_bwd(kp, fi, gk, acc);
+            dzi += __dmul_rn(2.0 * kern_diag_bwd(kp, fi, gk, acc), fi);
           } else {
-            double gfa, gfb;
-            ss_kern_bwd(kp, d, Zx + (size_t)i * d, fi, Zx + (size_t)j * d, kind ? zf[j] : 0.0, gk, acc, gfa, gfb);
-            dzi += 2.0 * gfa;
+            double ca, cb;
+            kern_entry_bwd(kp, d, Zx + (size_t)i * d, fi, Zx + (size_t)j * d, kind ? zf[j] : 0.0, gk, acc, ca, cb);
+            dzi += 2.0 * __dmul_rn(gk, ca);
           }
         }
         dzi = warp_sum(dzi);
         if (lane == 0) dzp[i] = dzi;
       }
-      ss_reduce_acc(acc, kp, d, red, th_pre);
+      ss_reduce_acc(acc, kp, red, th_pre);
     }
     // d loss / d raw theta and d loss / d raw noise of this layer
-    {
-      const int nth = theta_size(kind, d);
-      if (tid < nth && ldsc.g_raw_theta[tid])
-        ss_store(ldsc.g_raw_theta[tid], (th_rows[tid] + th_pre[tid]) * softplus_grad(*ldsc.raw_theta[tid]),
-                 D.accumulate);
-      if (tid == 64 && ldsc.g_raw_noise) {
-        const double s = sigmoid_fwd(*ldsc.raw_noise);
-        ss_store(ldsc.g_raw_noise, ds2_s[l] * (ldsc.noise_upper - ldsc.noise_lower) * s * (1.0 - s), D.accumulate);
-      }
-    }
+    store_raw_grads(tid, theta_size(kind, d), ldsc.raw_theta, ldsc.g_raw_theta, th_rows, th_pre, ldsc.raw_noise,
+                    ldsc.g_raw_noise, ldsc.noise_lower, ldsc.noise_upper, ds2_s[l], D.accumulate);
     __syncthreads();
   }
 
@@ -674,17 +572,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) small_step_kernel(const __grid_
       if (status_s[l] && status == 0.0) status = (double)(l + 1);
       retries = fmax(retries, (double)retries_s[l]);
     }
-    double* out = D.out;
-    const double loss = -(data - kl * kl_scale);
-    out[0] = loss;
-    out[1] = kl * kl_scale;
-    out[2] = data;
-    out[3] = status;
-    const bool finite = isfinite(loss);
-    if (status != 0.0 && out[4] == 0.0) out[4] = status;
-    if (!finite && status == 0.0) out[5] = 1.0;
-    out[6] = (status != 0.0 || !finite) ? 1.0 : 0.0;
-    out[7] = retries;
+    write_step_result(D.out, data, kl, kl_scale, status, retries);
   }
 }
 

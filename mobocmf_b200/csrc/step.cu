@@ -20,6 +20,77 @@ __device__ __forceinline__ double softplus_grad(double x) {
   return z / (z + 1.0);
 }
 __device__ __forceinline__ double sigmoid_fwd(double x) { return 1.0 / (1.0 + exp(-x)); }
+// Interval(lo, hi) constraint of the likelihood noise: lo + (hi - lo) sigmoid(raw), and g times its derivative
+__device__ __forceinline__ double interval_fwd(double lo, double hi, double raw) {
+  return lo + (hi - lo) * sigmoid_fwd(raw);
+}
+__device__ __forceinline__ double interval_bwd(double g, double lo, double hi, double raw) {
+  const double s = sigmoid_fwd(raw);
+  return g * (hi - lo) * s * (1.0 - s);
+}
+
+// ---- pieces shared by the fused step (the kernels below) and the single-kernel step (small_step.cu) ----------------
+// expected log-likelihood of one row (minibatch point with target y and fidelity fid, S rows per point) of layer
+// `layer` under noise s2:  returns data = w * -1/2 [ ((y - mu)^2 + max(v, 1e-10)) / s2 + log s2 + log 2 pi ],
+// w = [fid == layer] / S, and the derivatives of -data: ds2 by s2, dmu by mu, dv by v (0 for v < 1e-10)
+__device__ __forceinline__ double ell_row(double y, double fid, int layer, int S, double mu, double v, double s2,
+                                          double& ds2, double& dmu, double& dv) {
+  const double w = (fid == (double)layer) ? 1.0 / (double)S : 0.0;
+  const bool live = v >= kMinVariance;
+  const double vu = live ? v : kMinVariance;
+  const double res = y - mu;
+  const double q = res * res + vu;
+  ds2 = w * 0.5 * (1.0 / s2 - q / (s2 * s2));
+  dmu = -w * res / s2;
+  dv = live ? w * 0.5 / s2 : 0.0;
+  return w * -0.5 * (q / s2 + log(s2) + kLog2Pi);
+}
+
+// backward through the sample propagation f = mu + sqrt(max(v, 1e-10)) eps of the n rows base .. base + n - 1 of the
+// layer above that one row (mean mu, variance v) feeds, given their d / d f (row k reads eps[k % emod]; emod = 0:
+// eps[k]):  gmu = sum df,  gv = [v >= 1e-10] sum df eps / (2 sqrt(v))
+__device__ __forceinline__ void prop_bwd(const double* df, const double* eps, long long base, int n, int emod, double v,
+                                         double& gmu, double& gv) {
+  double s0 = 0.0, s1 = 0.0;
+  for (int k = 0; k < n; ++k) {
+    const double g = df[base + k];
+    s0 += g;
+    s1 = fma(g, eps[emod ? (base + k) % emod : base + k], s1);
+  }
+  gmu = s0;
+  gv = v >= kMinVariance ? s1 / (2.0 * sqrt(v)) : 0.0;
+}
+
+// out[0] loss, [1] KL * B / N, [2] data term, [3] status (first failed layer + 1, or 0), [4] sticky status,
+// [5] sticky "loss not finite", [6] this step is bad (Adam skips), [7] retries
+__device__ __forceinline__ void write_step_result(double* out, double data, double kl, double kl_scale, double status,
+                                                  double retries) {
+  const double loss = -(data - kl * kl_scale);
+  out[0] = loss;
+  out[1] = kl * kl_scale;
+  out[2] = data;
+  out[3] = status;
+  // the host reads these at its own pace (no per-step synchronisation): the first failure sticks, and the optimiser
+  // update of a bad step is skipped on the device (mobo_adam's skip flag)
+  const bool finite = isfinite(loss);
+  if (status != 0.0 && out[4] == 0.0) out[4] = status;
+  if (!finite && status == 0.0) out[5] = 1.0;
+  out[6] = (status != 0.0 || !finite) ? 1.0 : 0.0;
+  out[7] = retries;
+}
+
+__device__ __forceinline__ void store_grad(double* dst, double g, int accumulate) { *dst = accumulate ? *dst + g : g; }
+
+// d loss / d raw parameters of one layer through the constraint transforms (NULL destination: frozen): thread
+// tid < nth stores theta slot tid (softplus, d loss / d theta = dth_rows + dth_pre), thread 64 the noise (Interval)
+__device__ __forceinline__ void store_raw_grads(int tid, int nth, const double* const* raw_theta,
+                                                double* const* g_raw_theta, const double* dth_rows,
+                                                const double* dth_pre, const double* raw_noise, double* g_raw_noise,
+                                                double noise_lo, double noise_hi, double dnoise, int accumulate) {
+  if (tid < nth && g_raw_theta[tid])
+    store_grad(g_raw_theta[tid], (dth_rows[tid] + dth_pre[tid]) * softplus_grad(*raw_theta[tid]), accumulate);
+  if (tid == 64 && g_raw_noise) store_grad(g_raw_noise, interval_bwd(dnoise, noise_lo, noise_hi, *raw_noise), accumulate);
+}
 
 // ---- raw -> constrained parameters -----------------------------------------------------------------
 struct PrepArgs {
@@ -40,7 +111,7 @@ __global__ void step_prep_kernel(const __grid_constant__ PrepArgs a) {
   const int l = blockIdx.x, tid = threadIdx.x;
   const int nth = theta_size(l == 0 ? 0 : 1, a.d);
   if (tid < nth) a.theta[l][tid] = softplus_fwd(*a.raw_theta[l][tid]);
-  if (tid == 32) a.noise[l] = a.noise_lo[l] + (a.noise_hi[l] - a.noise_lo[l]) * sigmoid_fwd(*a.raw_noise[l]);
+  if (tid == 32) a.noise[l] = interval_fwd(a.noise_lo[l], a.noise_hi[l], *a.raw_noise[l]);
   if (tid == 33) a.clamp_count[l] = 0u;
   if (tid >= 64 && tid < 80) {
     a.gops_scal[l][tid - 64] = (tid - 64 == SC_KL) ? a.dkl : 0.0;
@@ -51,10 +122,8 @@ __global__ void step_prep_kernel(const __grid_constant__ PrepArgs a) {
 }
 
 // ---- expected log-likelihood of one layer's rows + the seed of its backward -------------------------
-//   row r of layer l belongs to minibatch point b = r / S_l; weight w = [fid_b == l] / S_l
-//   data  += w * -1/2 [ ((y - mu)^2 + max(v, 1e-10)) / s2 + log s2 + log 2 pi ]
-//   dmu    = d(-data)/dmu  + sum over the next layer's rows fed by this row of df
-//   dvar   = d(-data)/dv   + sum df * eps / (2 sqrt(max(v, 1e-10)))        (both v-paths gated by v >= 1e-10)
+//   row r of layer l belongs to minibatch point b = r / S_l:  data, dmu, dvar of ell_row, plus the next layer's
+//   share of dmu, dvar through its rows fed by this row (prop_bwd)
 // per-block partials (data, d(-data)/d s2) are folded in block order by step_finish_kernel.
 struct EllArgs {
   int layer;
@@ -78,27 +147,14 @@ __global__ void __launch_bounds__(ELL_THREADS) ell_kernel(const __grid_constant_
   double data = 0.0, ds2 = 0.0;
   if (r < a.R) {
     const long long b = r / a.S;
-    const double s2 = a.noise[a.layer];
-    const double w = (a.fid[b] == (double)a.layer) ? 1.0 / (double)a.S : 0.0;
-    const double mu = a.mu[r], v = a.var[r];
-    const bool live = v >= kMinVariance;
-    const double vu = live ? v : kMinVariance;
-    const double res = a.y[b] - mu;
-    const double q = res * res + vu;
-    data = w * -0.5 * (q / s2 + log(s2) + kLog2Pi);
-    ds2 = w * 0.5 * (1.0 / s2 - q / (s2 * s2));
-    double dmu = -w * res / s2;
-    double dv = live ? w * 0.5 / s2 : 0.0;
+    const double v = a.var[r];
+    double dmu, dv;
+    data = ell_row(a.y[b], a.fid[b], a.layer, a.S, a.mu[r], v, a.noise[a.layer], ds2, dmu, dv);
     if (a.df_next) {
-      double s0 = 0.0, s1 = 0.0;
-      const long long base = r * a.prep_next;
-      for (int k = 0; k < a.prep_next; ++k) {
-        const double g = a.df_next[base + k];
-        s0 += g;
-        s1 = fma(g, a.eps_next[base + k], s1);
-      }
-      dmu += s0;
-      if (live) dv += s1 / (2.0 * sqrt(vu));
+      double gmu, gv;
+      prop_bwd(a.df_next, a.eps_next, r * a.prep_next, a.prep_next, 0, v, gmu, gv);
+      dmu += gmu;
+      dv += gv;
     }
     a.dmu[r] = dmu;
     a.dvar[r] = dv;
@@ -159,36 +215,17 @@ __global__ void __launch_bounds__(256) step_finish_kernel(const __grid_constant_
       if (a.ops_scal[l][SC_STATUS] != 0.0 && status == 0.0) status = (double)(l + 1);
       retries = fmax(retries, a.ops_scal[l][SC_RETRIES]);
     }
-    const double loss = -(data - kl * a.kl_scale);
-    a.out[0] = loss;
-    a.out[1] = kl * a.kl_scale;
-    a.out[2] = data;
-    a.out[3] = status;
-    // the host reads these at its own pace (no per-step synchronisation): the first failure sticks, and the optimiser
-    // update of a bad step is skipped on the device (mobo_adam's skip flag)
-    const bool finite = isfinite(loss);
-    if (status != 0.0 && a.out[4] == 0.0) a.out[4] = status;
-    if (!finite && status == 0.0) a.out[5] = 1.0;
-    a.out[6] = (status != 0.0 || !finite) ? 1.0 : 0.0;
-    a.out[7] = retries;
+    write_step_result(a.out, data, kl, a.kl_scale, status, retries);
   }
   for (int l = 0; l < a.L; ++l) {
-    const int nth = theta_size(l == 0 ? 0 : 1, a.d);
-    if (tid < nth && a.g_raw_theta[l][tid]) {
-      const double g = (a.dtheta_rows[l][tid] + a.dtheta_pre[l][tid]) * softplus_grad(*a.raw_theta[l][tid]);
-      double* dst = a.g_raw_theta[l][tid];
-      *dst = a.accumulate ? *dst + g : g;
-    }
-    if (tid == 64 && a.g_raw_noise[l]) {
-      const double s = sigmoid_fwd(*a.raw_noise[l]);
-      const double g = sds2[l] * (a.noise_hi[l] - a.noise_lo[l]) * s * (1.0 - s);
-      *a.g_raw_noise[l] = a.accumulate ? *a.g_raw_noise[l] + g : g;
-    }
+    store_raw_grads(tid, theta_size(l == 0 ? 0 : 1, a.d), a.raw_theta[l], a.g_raw_theta[l], a.dtheta_rows[l],
+                    a.dtheta_pre[l], a.raw_noise[l], a.g_raw_noise[l], a.noise_lo[l], a.noise_hi[l], sds2[l],
+                    a.accumulate);
     if (a.g_m[l]) {
       for (int j = tid; j < a.M; j += 256) {
         double g = a.dm_pre[l][j];
         if (l + 1 < a.L) g += a.dzf_rows[l + 1][j] + a.dzf_pre[l + 1][j];
-        a.g_m[l][j] = a.accumulate ? a.g_m[l][j] + g : g;
+        store_grad(a.g_m[l] + j, g, a.accumulate);
       }
     }
   }
@@ -258,7 +295,7 @@ struct MomentArgs {
 __global__ void moment_kernel(const __grid_constant__ MomentArgs a) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
-  const double noise = a.noise_lo + (a.noise_hi - a.noise_lo) * sigmoid_fwd(*a.raw_noise);
+  const double noise = interval_fwd(a.noise_lo, a.noise_hi, *a.raw_noise);
   double s1 = 0.0, s2 = 0.0;
   for (int s = 0; s < a.S; ++s) {
     const long long r = a.tiled ? i * a.S + s : i;
@@ -291,8 +328,7 @@ constexpr int ACQ_THREADS = 256;
 __global__ void __launch_bounds__(ACQ_THREADS) acq_moment_bwd_kernel(const __grid_constant__ AcqMomentBwdArgs a) {
   __shared__ double red[ACQ_THREADS / 32];
   const long long i = (long long)blockIdx.x * ACQ_THREADS + threadIdx.x;
-  const double sg = sigmoid_fwd(*a.raw_noise);
-  const double noise = a.noise_lo + (a.noise_hi - a.noise_lo) * sg;
+  const double noise = interval_fwd(a.noise_lo, a.noise_hi, *a.raw_noise);
   double dn = 0.0;
   if (i < a.n) {
     const double gm = a.d_mu ? a.d_mu[i] : 0.0, gv = a.d_var ? a.d_var[i] : 0.0;
@@ -323,13 +359,12 @@ __global__ void __launch_bounds__(ACQ_THREADS) acq_moment_bwd_kernel(const __gri
   if (threadIdx.x == 0) {
     double s = 0.0;
     for (int w = 0; w < ACQ_THREADS / 32; ++w) s += red[w];
-    a.part[blockIdx.x] = s * (a.noise_hi - a.noise_lo) * sg * (1.0 - sg);
+    a.part[blockIdx.x] = interval_bwd(s, a.noise_lo, a.noise_hi, *a.raw_noise);
   }
 }
 
-// through the sample propagation f = mu_prev + sqrt(max(var_prev, 1e-10)) eps of the layer above, per row i of the
-// layer below (the rows i*prep .. i*prep+prep-1 above read it, row r reads eps[r % S]):
-//   dmu_prev[i] = sum_s df[i*prep+s],   dvar_prev[i] = [var_prev >= 1e-10] sum_s df eps / (2 sqrt(max(var_prev, 1e-10)))
+// through the sample propagation of the layer above (prop_bwd), per row i of the layer below: the rows
+// i*prep .. i*prep+prep-1 above read it, row r reads eps[r % S]
 __global__ void __launch_bounds__(ACQ_THREADS) acq_prop_bwd_kernel(const double* __restrict__ df,
                                                                    const double* __restrict__ var_prev,
                                                                    const double* __restrict__ eps, long long R_prev,
@@ -337,16 +372,7 @@ __global__ void __launch_bounds__(ACQ_THREADS) acq_prop_bwd_kernel(const double*
                                                                    double* __restrict__ dvar_prev) {
   const long long i = (long long)blockIdx.x * ACQ_THREADS + threadIdx.x;
   if (i >= R_prev) return;
-  const long long base = i * prep;
-  double s0 = 0.0, s1 = 0.0;
-  for (int s = 0; s < prep; ++s) {
-    const double g = df[base + s];
-    s0 += g;
-    s1 = fma(g, eps[(base + s) % S], s1);
-  }
-  const double v = var_prev[i];
-  dmu_prev[i] = s0;
-  dvar_prev[i] = v >= kMinVariance ? s1 / (2.0 * sqrt(v)) : 0.0;
+  prop_bwd(df, eps, i * prep, prep, S, var_prev[i], dmu_prev[i], dvar_prev[i]);
 }
 
 // dX[i][c] (+)= sum_l sum_{s < xrep_l} dxrow_l[i*xrep_l+s][c]: layer 0 first (xrep 1), then the layers above
